@@ -15,6 +15,7 @@ Workloads (BASELINE.json configs, SURVEY 8d):
   cfg5  --sweep: kernel-only on pre-inflated batches of 64 MB .. 8 GB
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config auto|cfg1|cfg2|cfg3|cfg4] [--records R]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 """
 import argparse
@@ -371,9 +372,55 @@ def all_tables(eng, dev):
     return c, s
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def result_arrays(eng):
+    """What a caller of the engine receives after bqc_finish, as float64 arrays that hold every value exactly: each
+    result table of each lane (per mate for the per-cycle fields, per q/k pair for the k-mer fields), the per-cycle mean
+    qualities, the KmerStream estimators, and the packed sketch words split into their low and high 32 bits (the words
+    are bit sets and do not fit a double's 53-bit mantissa)."""
+    from bamqc_b200.engine import FIELDS
+    n_qk = len(eng.klist) * len(eng.qlist)
+    out = {}
+    for lane in range(len(eng.lane_ids)):
+        for name, f in FIELDS.items():
+            if f >= FIELDS["SUMCOUNT"]:
+                subs = [(f"_qk{i}", i) for i in range(n_qk)]
+            elif f >= FIELDS["READLEN"]:
+                subs = [("_mate0", 0), ("_mate1", 1)]
+            else:
+                subs = [("", 0)]
+            for suffix, sub in subs:
+                t = eng.table(name, lane, sub)
+                if t.size and int(t.max()) >= 1 << 53:
+                    raise RuntimeError(f"lane {lane} {name}{suffix}: a count of 2**53 or more has no exact float64")
+                out[f"lane{lane}_{name}{suffix}"] = t.astype(np.float64)
+        for mate in (0, 1):
+            out[f"lane{lane}_avgqual_mean_mate{mate}"] = eng.avgqual(lane, mate).astype(np.float64)
+        for qk in range(n_qk):
+            est = eng.estimates(lane, qk)
+            out[f"lane{lane}_estimates_qk{qk}"] = np.array([est[k] for k in ("sumCount", "F0", "f1", "F2")], dtype=np.float64)
+            words = eng.sketch(lane, qk)
+            out[f"lane{lane}_sketch_qk{qk}"] = np.stack([words & np.uint64(0xFFFFFFFF), words >> np.uint64(32)], axis=1).astype(np.float64)
+    return out
+
+
+def dump_outputs(eng, out_dir):
+    """--dump-outputs: one <name>.npy per result array (result_arrays), at most DUMP_LIMIT_BYTES in all."""
+    arrays = result_arrays(eng)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of results, more than the {DUMP_LIMIT_BYTES} allowed")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"dumped {len(arrays)} result arrays ({total / 1e6:.1f} MB) to {out_dir}")
+
+
 def run_sweep(args):
     """cfg 5 of BASELINE.json: kernel-only throughput on pre-inflated record batches of 64 MB .. 8 GB resident in HBM
-    (one GPU, or one slice per rank under torchrun).  One JSON line per size: median and best of >= 10 repetitions,
+    (one GPU, or one slice per rank under torchrun).  One JSON line per size: median and best of --steps repetitions,
     CUDA events on the engine's stream.  Sizes below the L2 capacity are flagged (their inputs can sit in L2)."""
     import torch
     import torch.distributed as dist
@@ -398,7 +445,7 @@ def run_sweep(args):
             o = sub[lo:hi + 1]
             batches.append(eng.prepare(records[int(o[0]):int(o[-1])], o - o[0]))
         times = []
-        reps = max(10, args.steps)
+        reps = args.steps
         for it in range(args.warmup + reps):
             torch.cuda.synchronize(dev)
             if world > 1:
@@ -450,6 +497,9 @@ def run_b200(args):
     if need_gb > 0.8 * avail:
         f = 0.8 * avail / need_gb
         scaled = f"records per GPU scaled by {f:.2f}: {need_gb:.0f} GB of host memory needed, {avail:.0f} GB available"
+        if args.dump_outputs:  # dumps of two runs are comparable only if the arguments alone fix the inputs
+            raise SystemExit(f"--dump-outputs: {need_gb:.0f} GB of host memory needed, {avail:.0f} GB available; "
+                             "choose a smaller workload with --records instead of letting it be scaled down")
         log("warning: " + scaled)
         per_gpu = int(per_gpu * f)
         spec["records_per_gpu"], spec["records_total"] = per_gpu, per_gpu * world
@@ -525,6 +575,8 @@ def run_b200(args):
     total_records, total_bytes = float(tot[0].item()), float(tot[1].item())
     value = total_records * args.steps / (ms / 1e3)
     ref_tables = all_tables(eng, dev)
+    if args.dump_outputs and rank == 0:  # every rank holds the merged result after the last timed step
+        dump_outputs(eng, args.dump_outputs)
 
     # one more pass with the coverage kernels on the compute stream: exclusive device time per kernel family
     eng.profile_enable(2)
@@ -821,7 +873,13 @@ def main():
     ap.add_argument("--bgzf-level", type=int, default=6, help="zlib level of the synthetic BGZF input (samtools default: 6)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sweep", default="", help="cfg 5: comma separated batch sizes in MB per GPU (e.g. 64,256,1024,4096,8192); prints one line per size")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the results of the last one as DIR/<name>.npy (float64, exact)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.sweep):
+        ap.error("--dump-outputs applies to the timed path of --impl b200 without --sweep")
     if args.warmup < 3 and args.impl == "b200":
         log("note: fewer than 3 warm-up steps requested; timing rules ask for >= 3")
     if args.impl == "reference":
