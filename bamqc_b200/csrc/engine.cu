@@ -894,10 +894,14 @@ struct BatchLaunch {  // launch geometry shared by the coverage and the table ke
 // The reference's per-cycle String<>s grow with the longest read seen (src/QualityCheck.hpp:85-109); here the result
 // block has a per-cycle capacity, and a batch with a longer read moves every table to a larger layout before its
 // kernels are launched.  The limit is what k_stats can keep in shared memory (per-cycle rows of both mates).
+// A batch grows the capacity by at least half, so that a file of slowly increasing read lengths moves the block a few
+// times only; `exact` grows to pad8(need) instead, which is how two engines that grew along different steps are brought
+// to one layout before their blocks are added (bqc_merge_from, bqc_reserve_read_len).
 static const uint32_t kMaxReadLen = 1800;   // 2 mates x 9 padded per-cycle rows + 6 per-read histograms of that length: 216 KB of the 227 KB
-static int grow_read_len(bqc_engine* e, uint32_t need) {
+static int grow_read_len(bqc_engine* e, uint32_t need, bool exact = false) {
     if (need <= e->L.cyc || need > kMaxReadLen) return 0;   // longer: the kernel reports BQC_ERR_UNSUPPORTED
-    const uint32_t cyc2 = std::min<uint32_t>(pad8(kMaxReadLen), pad8(std::max<uint32_t>(need, e->L.cyc + e->L.cyc / 2)));
+    CU(cudaSetDevice(e->cfg.device));
+    const uint32_t cyc2 = exact ? pad8(need) : std::min<uint32_t>(pad8(kMaxReadLen), pad8(std::max<uint32_t>(need, e->L.cyc + e->L.cyc / 2)));
     const Layout A = e->L, Bn = make_layout(cyc2, A.isize1 - 1, A.n_qk, A.f2size, A.sk_size);
     std::vector<uint3> segs;
     auto seg = [&](uint32_t so, uint32_t d_o, uint32_t n) { segs.push_back(make_uint3(so, d_o, n)); };
@@ -1888,8 +1892,7 @@ extern "C" int bqc_reserve_read_len(bqc_engine* e, uint32_t n) {
     CU(cudaSetDevice(e->cfg.device));
     { int arc = drain_commits(e); if (arc) return arc; }
     if (n > kMaxReadLen) { set_error(e, "bqc_reserve_read_len: reads longer than %u are not supported", kMaxReadLen); return BQC_ERR_ARG; }
-    while (e->L.cyc < n) { const uint32_t before = e->L.cyc; int rc = grow_read_len(e, n); if (rc) return rc; if (e->L.cyc == before) break; }
-    return 0;
+    return grow_read_len(e, n, true);
 }
 extern "C" uint64_t bqc_counters_len(bqc_engine* e) { return (uint64_t)e->n_lanes * e->L.lane_stride; }
 extern "C" int bqc_counters_export(bqc_engine* e, void* dev) {
@@ -1929,8 +1932,10 @@ extern "C" int bqc_sketch_import_u8(bqc_engine* e, const void* dev) {
 }
 extern "C" int bqc_merge_from(bqc_engine* dst, bqc_engine* src) {
     bqc_engine* e = dst;
+    { int arc = drain_commits(dst); if (arc) return arc; }   // a batch still with the commit thread may grow either layout
+    { int arc = drain_commits(src); if (arc) { set_error(e, "bqc_merge_from: the source engine failed: %s", src->last_error.c_str()); return arc; } }
     if (dst->L.cyc != src->L.cyc) {  // one of them met a longer read: same layout first
-        int rc = dst->L.cyc < src->L.cyc ? grow_read_len(dst, src->L.cyc) : grow_read_len(src, dst->L.cyc);
+        int rc = dst->L.cyc < src->L.cyc ? grow_read_len(dst, src->L.cyc, true) : grow_read_len(src, dst->L.cyc, true);
         if (rc) return rc;
     }
     if (bqc_counters_len(dst) != bqc_counters_len(src) || bqc_sketch_len(dst) != bqc_sketch_len(src)) { set_error(e, "bqc_merge_from: engines differ in configuration"); return BQC_ERR_ARG; }

@@ -146,7 +146,9 @@ int bqc_finish(bqc_engine* e);
  * root.  dev_* pointers are device pointers on this engine's GPU. */
 uint64_t bqc_counters_len(bqc_engine* e);                 /* number of uint64 */
 /* The layout of the block depends on the per-cycle capacity, which grows with the longest read an engine has seen:
- * before exporting, bring every engine to the largest capacity of the group (all-reduce max of the capacities). */
+ * before exporting, bring every engine to the largest capacity of the group (all-reduce max of the capacities).
+ * bqc_reserve_read_len grows the capacity to exactly n rounded up to a multiple of 8 (never shrinks it), so an engine
+ * reserved to another engine's capacity has the same layout and bqc_counters_len. */
 uint32_t bqc_read_len_capacity(bqc_engine* e);
 int bqc_reserve_read_len(bqc_engine* e, uint32_t n);
 int bqc_counters_export(bqc_engine* e, void* dev_u64);    /* device -> device copy */

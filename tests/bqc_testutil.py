@@ -114,11 +114,114 @@ def run_engine(genome, lib_, records, offsets, out_path, chroms="chr1,chr2", isi
     return None
 
 
-def oracle_sketch(dump_path, n_sketches, size=32768, f2size=32768):
+def oracle_sketch_geometry(dump_path):
+    """[(size, F2size, sumCount)] of every sketch in the oracle's dump, in dump order (lanes in std::map order, then
+    q, then k): the `sketch_geometry` lines of oracle/bamqc_oracle.cpp (writeDump)."""
+    out = []
+    for line in open(dump_path):
+        f = line.split()
+        if f and f[0] == "sketch_geometry":
+            out.append((int(f[3]), int(f[4]), int(f[5])))
+    return out
+
+
+def oracle_sketch(dump_path, n_sketches=None):
+    """[(sketch table, F2 table)] of every sketch in the oracle's dump, sized by its `sketch_geometry` lines."""
+    geo = oracle_sketch_geometry(dump_path)
+    if n_sketches is not None:
+        assert len(geo) == n_sketches
     raw = np.fromfile(str(dump_path) + ".sketch", dtype=np.uint64)
-    per = 32 * size + f2size
-    assert raw.size == per * n_sketches
-    return [(raw[i * per:i * per + 32 * size], raw[i * per + 32 * size:(i + 1) * per]) for i in range(n_sketches)]
+    assert raw.size == sum(32 * size + f2size for size, f2size, _ in geo)
+    out, p = [], 0
+    for size, f2size, _ in geo:
+        out.append((raw[p:p + 32 * size], raw[p + 32 * size:p + 32 * size + f2size]))
+        p += 32 * size + f2size
+    return out
+
+
+def assert_sketches_equal(eng, dump_path, lane_ids, n_qk):
+    """Raw sketch, F2 table and sumCount of every (lane, q/k pair) of the engine equal to the oracle's dump."""
+    sk = oracle_sketch(dump_path, len(lane_ids) * n_qk)
+    geo = oracle_sketch_geometry(dump_path)
+    i = 0
+    for lane in sorted(range(len(lane_ids)), key=lambda l: lane_ids[l]):  # the oracle dumps lanes in std::map order
+        for qk in range(n_qk):
+            table, f2 = sk[i]
+            assert np.array_equal(eng.sketch(lane, qk), table), f"sketch table lane {lane} qk {qk}"
+            assert np.array_equal(eng.table("F2TABLE", lane, qk), f2), f"F2 table lane {lane} qk {qk}"
+            assert eng.estimates(lane, qk)["sumCount"] == geo[i][2], f"sumCount lane {lane} qk {qk}"
+            i += 1
+
+
+def kernel_names(fn):
+    """Run fn() under torch.profiler with CUDA activities; return (fn's result, the set of kernel names that ran).
+    Demangled names look like `void bqc::k_sketch32v2<640u>(bqc::EngineView, ...)`: match on substrings."""
+    import json
+    import tempfile
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        res = fn()
+        torch.cuda.synchronize()
+    with tempfile.TemporaryDirectory() as td:  # the trace lists every kernel, also those launched outside torch operators
+        path = os.path.join(td, "trace.json")
+        prof.export_chrome_trace(path)
+        events = json.load(open(path)).get("traceEvents", [])
+    return res, {e.get("name", "") for e in events if e.get("cat") == "kernel"}
+
+
+def assert_kernels(names, ran=(), not_ran=()):
+    for k in ran:
+        assert any(k in n for n in names), f"{k} did not run; kernels: {sorted(n for n in names if 'bqc::' in n)}"
+    for k in not_ran:
+        assert not any(k in n for n in names), f"{k} ran; kernels: {sorted(n for n in names if 'bqc::' in n)}"
+
+
+# Quality bytes where the kernels' unsigned forms of the reference's signed-char tests change behaviour: Q20 of the
+# triplet walk, the last ordinary cutoff (94 + 33 = 127), the sign flip of (char)(q + 33) at 95, and values far into
+# the negative range.  Bytes stay <= 222: from 223 on (char)(q + 33) wraps in the reference's own arithmetic.
+QUAL_EDGES = (19, 20, 93, 94, 95, 99, 100, 127, 128, 199, 200, 222)
+
+
+def mutate_qual(records, offsets, share=0.5, seed=0):
+    """Rewrite the QUAL bytes of about `share` of the records in place: per read either one edge value throughout (so a
+    cutoff at that value sees whole windows), runs of edge values, or independent draws from 0..222 weighted towards
+    the edges."""
+    rng = np.random.default_rng(seed)
+    edges = np.array(QUAL_EDGES, dtype=np.uint8)
+    for i in range(len(offsets) - 1):
+        if rng.random() >= share:
+            continue
+        o = int(offsets[i]) + 4
+        l_name = int(records[o + 8])
+        n_cig = int(records[o + 12]) | int(records[o + 13]) << 8
+        l_seq = int(records[o + 16]) | int(records[o + 17]) << 8 | int(records[o + 18]) << 16
+        qual = o + 32 + l_name + 4 * n_cig + (l_seq + 1) // 2
+        mode = rng.integers(3)
+        if mode == 0:
+            q = np.full(l_seq, rng.choice(edges), dtype=np.uint8)
+        elif mode == 1:
+            q = np.repeat(rng.choice(edges, size=l_seq // 16 + 1), 16)[:l_seq]
+        else:
+            q = np.where(rng.random(l_seq) < 0.5, rng.choice(edges, size=l_seq), rng.integers(0, 223, size=l_seq)).astype(np.uint8)
+        records[qual:qual + l_seq] = q
+
+
+def against_oracle(tmp_path, stream, opts=("-c", "chr1,chr2"), expect_rc=0):
+    """The drop-in command and the oracle on the same uncompressed BAM stream (golden genome): same exit status and,
+    on success, the same .bamqc."""
+    fasta = tmp_path / "g.fa"
+    golden_genome().write_fasta(fasta)
+    bam = tmp_path / "in.bam"
+    bam.write_bytes(stream)
+    o = subprocess.run([ensure_oracle(), "-r", str(fasta), "-o", str(tmp_path / "o.bamqc")] + list(opts) + [str(bam)], capture_output=True, text=True)
+    g = run_cli(["-r", fasta, "-o", tmp_path / "g.bamqc"] + list(opts) + [bam])
+    assert o.returncode == expect_rc, o.stderr
+    assert g.returncode == expect_rc, g.stderr + g.stdout
+    if expect_rc == 0:
+        diffs = diff_bamqc(tmp_path / "o.bamqc", tmp_path / "g.bamqc")
+        assert not diffs, "\n".join(diffs)
+    return o, g
 
 
 # ------------------------------------------------------------------------------------------------------

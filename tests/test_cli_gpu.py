@@ -29,19 +29,7 @@ def test_cli_reproduces_reference_bamqc(case, tmp_path):
     assert not diffs, "\n".join(diffs)
 
 
-def _against_oracle(tmp_path, stream, opts=("-c", "chr1,chr2"), expect_rc=0):
-    fasta = tmp_path / "g.fa"
-    util.golden_genome().write_fasta(fasta)
-    bam = tmp_path / "in.bam"
-    bam.write_bytes(stream)
-    o = subprocess.run([util.ensure_oracle(), "-r", str(fasta), "-o", str(tmp_path / "o.bamqc")] + list(opts) + [str(bam)], capture_output=True, text=True)
-    g = util.run_cli(["-r", fasta, "-o", tmp_path / "g.bamqc"] + list(opts) + [bam])
-    assert o.returncode == expect_rc, o.stderr
-    assert g.returncode == expect_rc, g.stderr + g.stdout
-    if expect_rc == 0:
-        diffs = util.diff_bamqc(tmp_path / "o.bamqc", tmp_path / "g.bamqc")
-        assert not diffs, "\n".join(diffs)
-    return o, g
+_against_oracle = util.against_oracle
 
 
 def test_empty_input(tmp_path):
