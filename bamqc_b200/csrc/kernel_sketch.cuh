@@ -9,6 +9,7 @@
 //   * the four 128-bit table lookups per base collapse into one 32-byte row indexed by (in, out):
 //     row = { H[in] ^ rotl_k(H[out]),  rotl_k(Ht[in]) ^ Ht[out] }.
 #pragma once
+#include "sketch_sched.h"
 
 namespace bqc {
 
@@ -222,11 +223,19 @@ __global__ void __launch_bounds__(kSketchThreads, 1) k_sketch32(EngineView E, Ba
 //   * the (in, out) pair table: a warp's lanes read different 32-byte rows that fall on the same banks -- 14 shared
 //     memory wavefronts per 16-byte load where 4 are the minimum, i.e. the LSU pipe busy half of the kernel's time
 //     and every hash step waiting ~3x longer for its row.
-// Here a read is processed in sub-chunks of 8 bases in two passes:
-//   pass 1  validity of the 8 bases (quality in [q, 94] as one unsigned range test, base != N; bases past the end of
-//           the read get quality 255) shifted into a 32-bit history: a base ends a window iff the history is all ones
-//           -> 8 emit bits; ONE warp prefix sum of the emit counts gives every lane its place in the warp's hash queue;
-//   pass 2  the 8 hash updates, unconditional; an emitted hash is one predicated 8-byte store at the lane's next slot.
+// Here a read is processed in sub-chunks of 8 bases, and a warp's 32 reads in two passes:
+//   pass 1  each lane walks its whole read, word-parallel (sketch_sched.h): the 8-base validity mask (quality in
+//           [q, 94] as one unsigned per-byte range test, base != N, inside the read) and a 32-bit validity history
+//           give the sub-chunks in which a window of 32 valid bases ends.  Only those are hashed: each run of them is
+//           cut into pieces of at most kPieceEmit sub-chunks, appended to a per-warp list in shared memory;
+//   pass 2  the lanes take the pieces 32 at a time.  A piece is hashed from zero state kPieceWarm sub-chunks before its
+//           first emitting one (exact: a window's hash depends on its 32 bases only), and per sub-chunk: the emit bits
+//           again, ONE warp prefix sum of the emit counts for every lane's place in the warp's hash queue, and the 8
+//           hash updates, unconditional; an emitted hash is one predicated 8-byte store at the lane's next slot.
+// With binned NovaSeq-like qualities and -q 17, about 9 % of the windows are valid and 5 of the 19 sub-chunks of a
+// 150 bp read emit; the pieces spread that work evenly over the lanes.  When the rounds of pieces would take the warp
+// no fewer steps than walking its reads from start to end (clean data: splitting only adds warm-up), or the list
+// overflows, the warp walks every lane's own read as one piece from sub-chunk 0 instead.
 // The hash tables are split by linearity -- row(in, out) = row_in(in) ^ row_out(out) -- into two 16-row tables that
 // are REPLICATED across the banks: a row holds 8 copies of its 16-byte part and 16 copies of its 8-byte part, lane l
 // reads copy l mod 8 (l mod 16), so the lanes of a quarter (half) warp never share a bank whatever they look up:
@@ -236,9 +245,13 @@ __global__ void __launch_bounds__(kSketchThreads, 1) k_sketch32(EngineView E, Ba
 // ------------------------------------------------------------------------------------------------
 static const uint32_t kSketchSub = 8;                                  // bases per sub-chunk
 static const uint32_t kSketchQueue2 = 31 + 32 * kSketchSub + 1;        // queue entries per warp: leftover + one sub-chunk of every lane
-// shared memory: [F2 table][in tables: 2 strands x 16 rows x 256 B][out tables: 2 strands x 16 rows x 128 B][zero: 16 x 128 B][queues]
+static const uint32_t kPlanSkip = 15;                                  // batches of 32 reads walked whole, unplanned, after a plan chose that
+static const uint32_t kPieceCap = 96;                                  // piece descriptors per warp (3 rounds; fits 1024 threads in 227 KB)
+// shared memory: [F2 table][in tables: 2 strands x 16 rows x 256 B][out tables: 2 strands x 16 rows x 128 B][zero: 16 x 128 B][queues][piece lists]
 static const uint32_t kSkIn = 2 * 16 * 256, kSkOut = 2 * 16 * 128, kSkZero = 16 * 128;
-__host__ __device__ inline uint32_t sketch32v2_smem(uint32_t f2size, uint32_t threads) { return f2size * 4u + kSkIn + kSkOut + kSkZero + (threads / 32u) * kSketchQueue2 * 8u; }
+__host__ __device__ inline uint32_t sketch32v2_smem(uint32_t f2size, uint32_t threads) {
+    return f2size * 4u + kSkIn + kSkOut + kSkZero + (threads / 32u) * (kSketchQueue2 * 8u + kPieceCap * 4u);
+}
 
 // exclusive prefix sum over the warp of a count in 0..8 without a dependent shuffle chain: one ballot per bit
 __device__ __forceinline__ uint32_t warp_prefix_small(uint32_t cnt, uint32_t lt_mask, uint32_t& total) {
@@ -256,6 +269,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_sketch32v2(EngineView E, BatchVi
     uint8_t* tout = tin + kSkIn;
     uint8_t* tzero = tout + kSkOut;
     uint64_t* queue = reinterpret_cast<uint64_t*>(tzero + kSkZero) + (threadIdx.x >> 5) * kSketchQueue2;
+    uint32_t* pieces = reinterpret_cast<uint32_t*>(reinterpret_cast<uint64_t*>(tzero + kSkZero) + (THREADS / 32u) * kSketchQueue2) + (threadIdx.x >> 5) * kPieceCap;
     for (uint32_t i = threadIdx.x; i < L.f2size; i += blockDim.x) sm[i] = 0;
     // in row (strand s, nibble n): copies of {a_lo = H[in].lo, b_lo = rotl_k(Ht''[in]).lo} then of {a_hi, b_hi} (see k_sketch32);
     // out row: copies of {rotl_k(H[out]).lo, Ht[out].lo}
@@ -291,6 +305,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_sketch32v2(EngineView E, BatchVi
     const uint32_t queue_s = (uint32_t)__cvta_generic_to_shared(queue);
     uint32_t qn = 0;                                 // queued hashes of this warp (uniform, < 32 between sub-chunks)
     SketchProbe2 probe = {kNone, 0u, 0u, kNone, 0u, 0u, 0u};
+    uint32_t plan_skip = 0;                          // batches of 32 reads still to walk whole without planning (uniform)
 
     auto probe_issue = [&](uint64_t hv) {            // StreamCounter::operator() (src/kmerstream/StreamCounter.hpp:67-93)
         probe.advance(sk);
@@ -324,92 +339,160 @@ __global__ void __launch_bounds__(THREADS, 1) k_sketch32v2(EngineView E, BatchVi
         const uint32_t s = act ? ((h.flag >> 4) & 1u) : 0u;
         const uint8_t* seqp = act ? h.p + h.o_seq : B.bytes;
         const uint8_t* qualp = act ? h.p + h.o_qual : B.bytes;
-        // this lane's copies: the row offset (nibble << 8, nibble << 7) is added to these shared-memory addresses
-        const uint32_t in_lo = sm_in + s * 4096u + (lane_id & 7u) * 16u, in_hi = sm_in + s * 4096u + 128u + (lane_id & 15u) * 8u;
-        const uint32_t out_lo = sm_out + s * 2048u + (lane_id & 7u) * 16u;
-        uint64_t hlo = 0, tlo = 0;
-        uint32_t hhi = 0, thi = 0;                    // top 32 bits of h.hi, low 32 bits of ht.hi
+        const uint32_t nsub = (maxL + kSketchSub - 1u) / kSketchSub;
+        auto align64 = [](uint64_t a, uint64_t b, uint32_t sh) { return (a >> sh) | ((b << 1) << (63u - sh)); };
+
+        // ---- pass 1: the emitting sub-chunks of this lane's read -> pieces in the warp's list
         // SEQ and QUAL are read as streams of ALIGNED 8-byte words, each loaded once and realigned in registers (one
         // SEQ word = 16 bases = two sub-chunks, one QUAL word per sub-chunk), two sub-chunks ahead of their use.  A lane
         // reads its own record, so every load touches 32 sectors per warp whatever its width: with the unaligned 4- and
         // 8-byte loads of the first version (two aligned loads each) a sector was fetched 16 times for SEQ and 8 times for
         // QUAL and the L1 data pipe was the busiest unit of the kernel (78 %, profiles/r2); now it is 4 times each.
-        const uint64_t* sA = reinterpret_cast<const uint64_t*>((uintptr_t)seqp & ~(uintptr_t)7);
-        const uint64_t* qA = reinterpret_cast<const uint64_t*>((uintptr_t)qualp & ~(uintptr_t)7);
-        const uint32_t ssh = ((uint32_t)(uintptr_t)seqp & 7u) * 8u, qsh = ((uint32_t)(uintptr_t)qualp & 7u) * 8u;
-        auto align64 = [](uint64_t a, uint64_t b, uint32_t sh) { return (a >> sh) | ((b << 1) << (63u - sh)); };
-        uint64_t A0 = __ldg(sA), A1 = __ldg(sA + 1);
-        uint64_t Q0 = __ldg(qA), Q1 = __ldg(qA + 1), Q2 = __ldg(qA + 2);
-        uint32_t lag0 = 0, lag1 = 0, lag2 = 0, lag3 = 0;  // SEQ words of the last 4 sub-chunks, oldest first (the base leaving a 32-window sits 4 words back)
-        uint32_t vh = 0;                              // validity of the last 32 bases, newest in bit 0
-        const uint32_t nsub = (maxL + kSketchSub - 1u) / kSketchSub;
-        auto sub_chunk = [&](const uint32_t c, const uint32_t seq_cur, uint64_t q_cur) {
-            // ---- pass 1: which of the 8 bases end a window of 32 valid bases
-            const uint32_t left = Ls > 8u * c ? Ls - 8u * c : 0u;           // bases of the read from here on
-            if (left < 8u) q_cur |= ~0ULL << (8u * left);                   // past the end: quality 255 = not valid
-            uint32_t emit = 0;
-#pragma unroll
-            for (uint32_t j = 0; j < 8; ++j) {
-                const uint32_t nin = (seq_cur >> (4u * (j ^ 1u))) & 15u;
-                const uint32_t q = (uint32_t)(q_cur >> (8u * j)) & 255u;
-                const bool valid = (q - q_lo_ok) <= q_span && nin != 15u;
-                vh += vh;
-                if (valid) vh |= 1u;
-                if (vh == 0xFFFFFFFFu) emit |= 1u << j;
-            }
-            uint32_t total;
-            const uint32_t excl = warp_prefix_small(__popc(emit), lt_mask, total);
-            uint32_t qp = queue_s + 8u * (qn + excl);                       // this lane's next queue slot
-            // ---- pass 2: the hash updates; h = rotl1(h) ^ H[in] ^ rotl_k(H[out]), ht = rotr1(ht ^ rotl_k(Ht[in]) ^ Ht[out])
-            const uint32_t outw = lag0;
-            const uint32_t o_base = c >= 4u ? out_lo : zero_lo;
-#pragma unroll
-            for (uint32_t j = 0; j < 8; ++j) {
-                const uint32_t sh = 4u * (j ^ 1u);
-                const uint32_t ni = sh >= 8u ? (seq_cur >> (sh - 8u)) & 0xF00u : (seq_cur << (8u - sh)) & 0xF00u;   // nibble << 8
-                const uint32_t no = sh >= 7u ? (outw >> (sh - 7u)) & 0x780u : (outw << (7u - sh)) & 0x780u;         // nibble << 7
-                uint64_t a_lo, b_lo, oa_lo, ob_lo;
-                uint32_t a_hi, b_hi;
-                asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(a_lo), "=l"(b_lo) : "r"(in_lo + ni));
-                asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(a_hi), "=r"(b_hi) : "r"(in_hi + ni));
-                asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(oa_lo), "=l"(ob_lo) : "r"(o_base + no));
-                hlo = ((hlo << 1) | (uint64_t)(hhi >> 31)) ^ a_lo ^ oa_lo;
-                hhi = (hhi << 1) ^ a_hi;
-                const uint64_t xl = tlo ^ b_lo ^ ob_lo;
-                const uint32_t xh = thi ^ b_hi;
-                tlo = (xl >> 1) | ((uint64_t)xh << 63);
-                thi = xh >> 1;
-                if ((emit >> j) & 1u) {
-                    const uint64_t hv = hlo ^ tlo;
-                    asm volatile("st.shared.u64 [%0], %1;" ::"r"(qp), "l"(hv) : "memory");
-                    qp += 8u;
+        // A warp whose last plan was the whole-read walk skips the next kPlanSkip plans and walks whole reads straight
+        // away: on clean data (every window valid) or where the list overflows (long reads), pass 1 would cost its
+        // walk over the reads and save nothing; the quality profile of neighbouring reads changes slowly.
+        uint32_t npieces = 0;                         // pieces of the warp (uniform; > kPieceCap: the list overflowed)
+        const bool plan = plan_skip == 0u && nsub <= kPieceMaxSub;
+        if (plan) {
+            __syncwarp();                             // the list of the previous 32 reads has been read
+            const uint64_t* sA = reinterpret_cast<const uint64_t*>((uintptr_t)seqp & ~(uintptr_t)7);
+            const uint64_t* qA = reinterpret_cast<const uint64_t*>((uintptr_t)qualp & ~(uintptr_t)7);
+            const uint32_t ssh = ((uint32_t)(uintptr_t)seqp & 7u) * 8u, qsh = ((uint32_t)(uintptr_t)qualp & 7u) * 8u;
+            uint64_t A0 = __ldg(sA), A1 = __ldg(sA + 1);
+            uint64_t Q0 = __ldg(qA), Q1 = __ldg(qA + 1), Q2 = __ldg(qA + 2);
+            uint32_t hv = 0;
+            PieceSplitter split = {0u, 0u};
+            auto append = [&](bool close, uint32_t p_es, uint32_t p_end) {
+                const uint32_t b = __ballot_sync(0xFFFFFFFFu, close);
+                if (b) {  // warp-uniform
+                    const uint32_t i = npieces + __popc(b & lt_mask);
+                    if (close && i < kPieceCap) pieces[i] = piece_desc(lane_id, p_es, p_end);
+                    npieces += __popc(b);
                 }
+            };
+            // 16 bases (sub-chunks c, c + 1) per step; sub-chunk nsub, when c + 1 == nsub, is past every read: it emits
+            // nothing and closes what is open, as the flush would
+            for (uint32_t c = 0; c < nsub; c += 2u) {
+                const uint64_t A2 = __ldg(sA + (c >> 1) + 2u);              // reads past a short record stay inside the padded batch
+                const uint64_t Q3 = __ldg(qA + c + 3u), Q4 = __ldg(qA + c + 4u);
+                const uint32_t e = sketch_emit16(hv, sketch_valid16(align64(Q0, Q1, qsh), align64(Q1, Q2, qsh), align64(A0, A1, ssh), c, Ls, q_lo_ok, q_span));
+                uint32_t p_es = 0, p_end = 0;
+                bool close = split.step(c, (e & 0xFFu) != 0u, p_es, p_end);
+                close |= split.step(c + 1u, (e >> 8) != 0u, p_es, p_end);
+                append(close, p_es, p_end);
+                A0 = A1; A1 = A2;
+                Q0 = Q2; Q1 = Q3; Q2 = Q4;
             }
-            lag0 = lag1; lag1 = lag2; lag2 = lag3; lag3 = seq_cur;
-            if (total) {  // warp-uniform
-                __syncwarp();
-                warp_count += total;
-                const uint32_t have = qn + total;
-                uint32_t done = 0;
-                for (; done + 32u <= have; done += 32u) probe_issue(queue[done + lane_id]);
-                const uint32_t rest = have - done;
-                if (done && rest) {                                         // what is left moves to the front of the queue
-                    const uint64_t v = lane_id < rest ? queue[done + lane_id] : 0ull;
+            uint32_t p_es = 0, p_end = 0;
+            const bool close = split.flush(nsub, p_es, p_end);
+            append(close, p_es, p_end);
+            __syncwarp();
+        }
+        // rounds of 32 pieces take the longest piece of each round (pieces in the order they were found: longest-first
+        // would save about 6 % of the steps at -q 17 in a model of the synthetic library); walking the reads from
+        // sub-chunk 0 takes nsub steps
+        uint32_t split_steps = 0;
+        const uint32_t split_rounds = (npieces + 31u) / 32u;
+        if (plan && npieces <= kPieceCap) {
+            for (uint32_t r = 0; r < split_rounds; ++r) {
+                const uint32_t i = r * 32u + lane_id;
+                const uint32_t d = i < npieces ? pieces[i] : 0u;
+                split_steps += __reduce_max_sync(0xFFFFFFFFu, (d >> 16) - piece_warm_start((d >> 8) & 255u));
+            }
+        }
+        const bool use_pieces = plan && npieces <= kPieceCap && split_steps < nsub;
+        if (plan) plan_skip = use_pieces ? 0u : kPlanSkip;
+        else if (plan_skip) --plan_skip;
+        const uint32_t nrounds = use_pieces ? split_rounds : 1u;
+
+        // ---- pass 2: the hash updates, one piece per lane and round
+        for (uint32_t r = 0; r < nrounds; ++r) {
+            uint32_t own = lane_id, es = 0, end = use_pieces ? 0u : nsub;   // unsplit: the lane's own read, sub-chunks 0..nsub-1
+            if (use_pieces && r * 32u + lane_id < npieces) {
+                const uint32_t d = pieces[r * 32u + lane_id];
+                own = d & 31u;
+                es = (d >> 8) & 255u;
+                end = d >> 16;
+            }
+            const uint32_t ws = piece_warm_start(es);
+            const uint32_t steps = __reduce_max_sync(0xFFFFFFFFu, end - ws);
+            // the owning lane's read
+            const uint8_t* pseq = reinterpret_cast<const uint8_t*>(__shfl_sync(0xFFFFFFFFu, (unsigned long long)(uintptr_t)seqp, own));
+            const uint8_t* pqual = reinterpret_cast<const uint8_t*>(__shfl_sync(0xFFFFFFFFu, (unsigned long long)(uintptr_t)qualp, own));
+            const uint32_t pLs = __shfl_sync(0xFFFFFFFFu, Ls, own), ps = __shfl_sync(0xFFFFFFFFu, s, own);
+            // this lane's copies: the row offset (nibble << 8, nibble << 7) is added to these shared-memory addresses
+            const uint32_t in_lo = sm_in + ps * 4096u + (lane_id & 7u) * 16u, in_hi = sm_in + ps * 4096u + 128u + (lane_id & 15u) * 8u;
+            const uint32_t out_lo = sm_out + ps * 2048u + (lane_id & 7u) * 16u;
+            // a piece starts at any sub-chunk: SEQ as aligned 4-byte words (one per sub-chunk), QUAL as aligned 8-byte words,
+            // realigned in registers and loaded one sub-chunk ahead; never past word end + 1 of the piece's read.  One
+            // 4-byte SEQ load per sub-chunk instead of an 8-byte one per two keeps a piece free to start at an odd
+            // sub-chunk; with pass 1 that is more global loads per read than one walk, but each hashed sub-chunk saved
+            // drops 24 table LDS (80 shared wavefronts) from the same L1 pipe
+            const uint32_t* sW = reinterpret_cast<const uint32_t*>((uintptr_t)pseq & ~(uintptr_t)3);
+            const uint64_t* qA = reinterpret_cast<const uint64_t*>((uintptr_t)pqual & ~(uintptr_t)7);
+            const uint32_t ssh = ((uint32_t)(uintptr_t)pseq & 3u) * 8u, qsh = ((uint32_t)(uintptr_t)pqual & 7u) * 8u;
+            uint32_t S0 = __ldg(sW + ws), S1 = __ldg(sW + ws + 1u);
+            uint64_t Q0 = __ldg(qA + ws), Q1 = __ldg(qA + ws + 1u);
+            uint64_t hlo = 0, tlo = 0;
+            uint32_t hhi = 0, thi = 0;                // top 32 bits of h.hi, low 32 bits of ht.hi
+            uint32_t lag0 = 0, lag1 = 0, lag2 = 0, lag3 = 0;  // SEQ words of the last 4 sub-chunks, oldest first (the base leaving a 32-window sits 4 words back)
+            uint32_t hv = 0;                          // validity of the last 32 bases, oldest in bit 0
+            for (uint32_t t = 0; t < steps; ++t) {
+                const uint32_t c = ws + t;
+                const uint32_t nx = min(c + 2u, end + 1u);
+                const uint32_t S2 = __ldg(sW + nx);
+                const uint64_t Q2 = __ldg(qA + nx);
+                const uint32_t seq_cur = __funnelshift_r(S0, S1, ssh);
+                uint32_t emit = sketch_emit8(hv, sketch_valid8(align64(Q0, Q1, qsh), seq_cur, c, pLs, q_lo_ok, q_span));
+                if (c < es || c >= end) emit = 0u;    // warm-up (hashed by the previous piece) or past the piece
+                uint32_t total;
+                const uint32_t excl = warp_prefix_small(__popc(emit), lt_mask, total);
+                uint32_t qp = queue_s + 8u * (qn + excl);                   // this lane's next queue slot
+                // h = rotl1(h) ^ H[in] ^ rotl_k(H[out]), ht = rotr1(ht ^ rotl_k(Ht[in]) ^ Ht[out]); the first 32 bases
+                // after the (re)start look up the all-zero `out` table
+                const uint32_t outw = lag0;
+                const uint32_t o_base = c >= ws + 4u ? out_lo : zero_lo;
+#pragma unroll
+                for (uint32_t j = 0; j < 8; ++j) {
+                    const uint32_t sh = 4u * (j ^ 1u);
+                    const uint32_t ni = sh >= 8u ? (seq_cur >> (sh - 8u)) & 0xF00u : (seq_cur << (8u - sh)) & 0xF00u;   // nibble << 8
+                    const uint32_t no = sh >= 7u ? (outw >> (sh - 7u)) & 0x780u : (outw << (7u - sh)) & 0x780u;         // nibble << 7
+                    uint64_t a_lo, b_lo, oa_lo, ob_lo;
+                    uint32_t a_hi, b_hi;
+                    asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(a_lo), "=l"(b_lo) : "r"(in_lo + ni));
+                    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(a_hi), "=r"(b_hi) : "r"(in_hi + ni));
+                    asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(oa_lo), "=l"(ob_lo) : "r"(o_base + no));
+                    hlo = ((hlo << 1) | (uint64_t)(hhi >> 31)) ^ a_lo ^ oa_lo;
+                    hhi = (hhi << 1) ^ a_hi;
+                    const uint64_t xl = tlo ^ b_lo ^ ob_lo;
+                    const uint32_t xh = thi ^ b_hi;
+                    tlo = (xl >> 1) | ((uint64_t)xh << 63);
+                    thi = xh >> 1;
+                    if ((emit >> j) & 1u) {
+                        const uint64_t hval = hlo ^ tlo;
+                        asm volatile("st.shared.u64 [%0], %1;" ::"r"(qp), "l"(hval) : "memory");
+                        qp += 8u;
+                    }
+                }
+                lag0 = lag1; lag1 = lag2; lag2 = lag3; lag3 = seq_cur;
+                S0 = S1; S1 = S2;
+                Q0 = Q1; Q1 = Q2;
+                if (total) {  // warp-uniform
                     __syncwarp();
-                    if (lane_id < rest) queue[lane_id] = v;
+                    warp_count += total;
+                    const uint32_t have = qn + total;
+                    uint32_t done = 0;
+                    for (; done + 32u <= have; done += 32u) probe_issue(queue[done + lane_id]);
+                    const uint32_t rest = have - done;
+                    if (done && rest) {                                     // what is left moves to the front of the queue
+                        const uint64_t v = lane_id < rest ? queue[done + lane_id] : 0ull;
+                        __syncwarp();
+                        if (lane_id < rest) queue[lane_id] = v;
+                    }
+                    qn = rest;
+                    __syncwarp();
                 }
-                qn = rest;
-                __syncwarp();
             }
-        };
-        for (uint32_t c = 0; c < nsub; c += 2u) {
-            const uint64_t A2 = __ldg(sA + (c >> 1) + 2u);                  // reads past a short record stay inside the padded batch
-            const uint64_t Q3 = __ldg(qA + c + 3u), Q4 = __ldg(qA + c + 4u);
-            const uint64_t sv = align64(A0, A1, ssh);
-            sub_chunk(c, (uint32_t)sv, align64(Q0, Q1, qsh));
-            if (c + 1u < nsub) sub_chunk(c + 1u, (uint32_t)(sv >> 32), align64(Q1, Q2, qsh));
-            A0 = A1; A1 = A2;
-            Q0 = Q2; Q1 = Q3; Q2 = Q4;
         }
     }
     __syncwarp();
