@@ -116,6 +116,9 @@ PROTOTYPES = {
     "bqc_cov_shard_boundary": (ctypes.c_int, [_vp, _P(bqc_cov_shard)]),
     "bqc_cov_shard_function": (ctypes.c_int, [_vp, _i32, _i32, _u32, _vp]),
     "bqc_cov_shard_run": (ctypes.c_int, [_vp, _i32, _i32, _u32, _u32, _P(bqc_cov_shard)]),
+    "bqc_cov_shard_boundary_lane": (ctypes.c_int, [_vp, _i32, _P(bqc_cov_shard)]),
+    "bqc_cov_shard_function_lane": (ctypes.c_int, [_vp, _i32, _i32, _i32, _u32, _vp]),
+    "bqc_cov_shard_run_lane": (ctypes.c_int, [_vp, _i32, _i32, _i32, _u32, _u32, _P(bqc_cov_shard)]),
     "bqc_cov_shards_combine": (None, [_vp, _i32, _vp]),
     "bqc_cov_apply": (_u32, [_vp, _u32]),
     "bqc_poscov_adjust": (ctypes.c_int, [_vp, _i32, _vp]),

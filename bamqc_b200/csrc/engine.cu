@@ -169,9 +169,11 @@ struct bqc_engine {
     bool cov_head_piece = false;       // shard mode of the FIRST piece of a stream: its entry state is known, so it runs like a
                                        // normal engine; only the end-of-run flush is left to bqc_cov_shards_combine
     uint64_t cov_acc_bound = 0;        // shard mode: upper bound of the records collected so far
+    uint8_t* d_cov_lq = nullptr;       // shard mode, several lanes: the collected records grouped by lane (rid, begin, interval),
+    std::vector<uint32_t> cov_lane_range;  // ... lane l owns [range[l], range[l + 1]); empty until cov_lane_split, freed by bqc_reset
     uint16_t* d_cov_fn = nullptr;      // shard mode: [1024] shard function; [2048 int32] head
     uint64_t cov_ctl_bytes = 0;        // tickets + look-back states at the front of the scratch (zeroed per launch group)
-    CovScratch cov_scratch;
+    CovScratch cov_scratch = {};
     unsigned long long* d_error = nullptr;
     const uint32_t** d_ref = nullptr;
     uint64_t* d_ref_len = nullptr;
@@ -364,6 +366,7 @@ extern "C" void bqc_destroy(bqc_engine* e) {
     cudaFree(e->d_cov_d);
     cudaFree(e->d_cov_scratch);
     cudaFree(e->d_cov_q);
+    cudaFree(e->d_cov_lq);
     cudaFree(e->d_cov_fn);
     cudaFree(e->d_tab_tickets);
     cudaFree(e->d_error);
@@ -427,6 +430,9 @@ extern "C" int bqc_reset(bqc_engine* e) {
     CU(cudaStreamSynchronize(e->compute));  // the coverage stream starts from a clean state
     e->records_seen = 0;
     e->cov_acc_bound = 0;
+    cudaFree(e->d_cov_lq);
+    e->d_cov_lq = nullptr;
+    e->cov_lane_range.clear();
     e->finished = false;
     e->have_results = false;
     e->host_error.code = 0;
@@ -814,15 +820,19 @@ extern "C" int bqc_profile_read(bqc_engine* e, double ms_out[12], uint64_t n_out
 // Scratch of the coverage kernels for a batch of up to n records: one allocation, grown on demand (rare: the first
 // batch, or a larger resident batch).  Layout: control words that are zeroed before every launch group (tickets,
 // look-back states), then the per-record and per-block arrays.  The compact records themselves live in their own
-// allocation because shard mode keeps collecting them over the whole run (`keep` entries survive a growth).
+// allocation because shard mode keeps collecting them over the whole run (`keep` entries survive a growth).  With
+// several read groups a one-byte lane tag per record follows the four arrays.
 static int ensure_cov_q(bqc_engine* e, uint64_t n_records, uint64_t keep) {
     if (n_records <= e->cov_q_cap && e->d_cov_q) return 0;
     const uint64_t N = std::max<uint64_t>(n_records + n_records / 4, 1u << 16);
+    const uint64_t tag = e->n_lanes > 1 ? N : 0;
     uint8_t* m = nullptr;
     CU(cudaStreamSynchronize(e->covs));
-    CU(cudaMalloc(&m, N * 16));
-    if (e->d_cov_q && keep)
+    CU(cudaMalloc(&m, N * 16 + tag));
+    if (e->d_cov_q && keep) {
         for (int a = 0; a < 4; ++a) CU(cudaMemcpy(m + (uint64_t)a * N * 4, e->d_cov_q + (uint64_t)a * e->cov_q_cap * 4, keep * 4, cudaMemcpyDeviceToDevice));
+        if (tag) CU(cudaMemcpy(m + N * 16, e->d_cov_q + e->cov_q_cap * 16, keep, cudaMemcpyDeviceToDevice));
+    }
     cudaFree(e->d_cov_q);
     e->d_cov_q = m;
     e->cov_q_cap = N;
@@ -831,6 +841,7 @@ static int ensure_cov_q(bqc_engine* e, uint64_t n_records, uint64_t keep) {
     S.q_b = (uint32_t*)(m + N * 4);
     S.q_iv = (uint32_t*)(m + N * 8);
     S.q_rec = (uint32_t*)(m + N * 12);
+    S.q_lane = tag ? m + N * 16 : nullptr;
     return 0;
 }
 static int ensure_cov_scratch(bqc_engine* e, uint64_t n_records) {
@@ -975,9 +986,8 @@ static int batch_launch_setup(bqc_engine* e, const DeviceBatch& d, BatchLaunch& 
 }
 
 // The anchor recurrence, the virtual coordinates and the depth histogram of the records collected in the compact
-// arrays (a batch, or a whole shard), from the state in CovCarry; n_bound >= the number of compact records.
-static int launch_cov_resolve(bqc_engine* e, uint32_t lane, const BatchView& B, uint64_t n_bound, bool tables_done) {
-    const CovScratch& S = e->cov_scratch;
+// arrays of S (a batch, or a whole shard), from the state in CovCarry; n_bound >= the number of compact records.
+static int launch_cov_resolve(bqc_engine* e, uint32_t lane, const CovScratch& S, const BatchView& B, uint64_t n_bound, bool tables_done) {
     cudaStream_t cs = cov_stream(e);
     CovCarry* carry = e->d_cov_carry + lane;
     int32_t* cd = e->d_cov_d + (uint64_t)lane * 2 * kCovD;
@@ -1014,14 +1024,23 @@ static int launch_cov(bqc_engine* e, const DeviceBatch& d, const BatchLaunch& BL
         B.cycb = BL.cycb;
         B.first_record = d.first_record;
         const uint32_t nprep = (uint32_t)((n + kCovPrepTile - 1) / kCovPrepTile);
+        const int gprep = (int)std::min<uint32_t>(nprep, (uint32_t)e->n_sm * 2u);
         ProfScope prof(e, 3, cs);
-        for (uint32_t lane = 0; lane < e->n_lanes; ++lane) {
+        // shard mode with several read groups: one pass over all lanes into one tagged queue (its running total in
+        // carry[0].nq), grouped by lane when the run has ended (cov_lane_split)
+        const bool tagged = e->cov_deferred && e->n_lanes > 1;
+        if (tagged) {
+            CU(cudaMemsetAsync(e->d_cov_scratch, 0, e->cov_ctl_bytes, cs));
+            k_cov_prep<true><<<gprep, kCovPrepThreads, 0, cs>>>(BL.E, B, 0, S, e->d_cov_carry, 1u);
+            e->launches += 1;
+        }
+        for (uint32_t lane = 0; lane < e->n_lanes && !tagged; ++lane) {
             CovCarry* carry = e->d_cov_carry + lane;
             CU(cudaMemsetAsync(e->d_cov_scratch, 0, e->cov_ctl_bytes, cs));
-            k_cov_prep<<<(int)std::min<uint32_t>(nprep, (uint32_t)e->n_sm * 2u), kCovPrepThreads, 0, cs>>>(BL.E, B, lane, S, carry, e->cov_deferred ? 1u : 0u);
+            k_cov_prep<false><<<gprep, kCovPrepThreads, 0, cs>>>(BL.E, B, lane, S, carry, e->cov_deferred ? 1u : 0u);
             e->launches += 1;
             if (e->cov_deferred) continue;
-            rc = launch_cov_resolve(e, lane, B, n, false);
+            rc = launch_cov_resolve(e, lane, S, B, n, false);
             if (rc) return rc;
             k_cov_carry<<<1, 1024, 0, cs>>>(B, S, carry, e->d_cov_d + (uint64_t)lane * 2 * kCovD);
             e->launches += 1;
@@ -1744,14 +1763,47 @@ extern "C" int bqc_finish(bqc_engine* e) {
 // one record stream cut across several engines: the coverage statistic (include/bamqc_b200.h, cov_math.h "Shards")
 // ------------------------------------------------------------------------------------------------
 extern "C" int bqc_cov_defer(bqc_engine* e, int on) {
-    if (on && e->n_lanes != 1) { set_error(e, "bqc_cov_defer: shard mode supports a single read group"); return BQC_ERR_ARG; }
     if (e->records_seen || e->cov_acc_bound) { set_error(e, "bqc_cov_defer: call it right after bqc_reset"); return BQC_ERR_ARG; }
     e->cov_deferred = on == 1;
     e->cov_head_piece = on == 2;
     return 0;
 }
 
-static int cov_shard_sync(bqc_engine* e, uint32_t& nq) {
+// Shard mode with several read groups collects every lane's records in one queue, in file order, each tagged with its
+// lane (launch_cov), so that the queue needs no more room than with one lane.  The first shard call after the run
+// groups it by lane: k_lane_partition over the tags (lane by lane, file order inside a lane), then one gather into a
+// copy whose lane l owns [cov_lane_range[l], cov_lane_range[l + 1]).  Kept until bqc_reset.  n: the records collected.
+static int cov_lane_split(bqc_engine* e, uint32_t n) {
+    const uint64_t N = std::max<uint32_t>(n, 1u);
+    const uint64_t o_range = N * 16, o_lb = (o_range + (e->n_lanes + 1) * 4 + 7) & ~7ull, lb_bytes = (N / 1024 + 4) * 8;
+    cudaFree(e->d_cov_lq);
+    CU(cudaMalloc(&e->d_cov_lq, o_lb + lb_bytes));
+    uint8_t* m = e->d_cov_lq;
+    uint32_t* index = (uint32_t*)(m + N * 12);
+    uint32_t* range = (uint32_t*)(m + o_range);
+    unsigned long long* lb = (unsigned long long*)(m + o_lb);
+    cudaStream_t st = cov_stream(e);
+    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((n + 1023) / 1024, (uint64_t)e->n_sm * 2));
+    ProfScope prof(e, 3, st);
+    for (uint32_t lane = 0; lane < e->n_lanes; ++lane) {
+        CU(cudaMemsetAsync(lb, 0, lb_bytes, st));
+        k_lane_partition<<<grid, 1024, 0, st>>>(e->cov_scratch.q_lane, nullptr, n, lane, index, range, lb + 1, (uint32_t*)lb);
+    }
+    if (n) k_cov_lane_gather<<<grid, 1024, 0, st>>>(e->cov_scratch, index, n, (int32_t*)m, (uint32_t*)(m + N * 4), (uint32_t*)(m + N * 8));
+    e->launches += e->n_lanes + (n ? 1u : 0u);
+    CU(cudaGetLastError());
+    std::vector<uint32_t> r(e->n_lanes + 1);
+    CU(cudaMemcpyAsync(r.data(), range, (e->n_lanes + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    e->cov_lane_range.swap(r);
+    return 0;
+}
+
+// Every shard call: checks its arguments, synchronises the engine and returns how many records of `lane` were
+// collected (grouping them by lane first, see cov_lane_split).
+static int cov_shard_sync(bqc_engine* e, const char* fn, int32_t lane, uint32_t& nq) {
+    if (!e->cov_deferred && !e->cov_head_piece) { set_error(e, "%s: engine is not in shard mode (bqc_cov_defer)", fn); return BQC_ERR_ARG; }
+    if (lane < 0 || (uint32_t)lane >= e->n_lanes) { set_error(e, "%s: bad lane", fn); return BQC_ERR_ARG; }
     CU(cudaSetDevice(e->cfg.device));
     { int arc = drain_commits(e); if (arc) return arc; }
     CU(cudaStreamSynchronize(e->compute));
@@ -1759,18 +1811,43 @@ static int cov_shard_sync(bqc_engine* e, uint32_t& nq) {
     CovCarry c;
     CU(cudaMemcpy(&c, e->d_cov_carry, sizeof(c), cudaMemcpyDeviceToHost));
     nq = c.nq;
+    if (e->cov_deferred && e->n_lanes > 1) {
+        if (e->cov_lane_range.empty()) { int rc = cov_lane_split(e, c.nq); if (rc) return rc; }
+        nq = e->cov_lane_range[lane + 1] - e->cov_lane_range[lane];
+    }
     return 0;
 }
 
-extern "C" int bqc_cov_shard_boundary(bqc_engine* e, bqc_cov_shard* out) {
+// The compact records of `lane` as the resolving kernels see them: the whole queue with one lane, the lane's segment
+// of the grouped copy with several (no record index: a record that needs its bytes again is refused in shard mode).
+static CovScratch cov_lane_scratch(bqc_engine* e, int32_t lane) {
+    CovScratch S = e->cov_scratch;
+    if (e->cov_deferred && e->n_lanes > 1) {
+        const uint64_t N = std::max<uint32_t>(e->cov_lane_range.back(), 1u), a = e->cov_lane_range[lane];
+        S.q_rid = (int32_t*)e->d_cov_lq + a;
+        S.q_b = (uint32_t*)(e->d_cov_lq + N * 4) + a;
+        S.q_iv = (uint32_t*)(e->d_cov_lq + N * 8) + a;
+        S.q_rec = nullptr;
+        S.q_lane = nullptr;
+    }
+    return S;
+}
+
+// With several lanes the carry of a lane does not hold the lane's record count: set it before its records are resolved.
+static int cov_lane_set_nq(bqc_engine* e, int32_t lane, uint32_t nq) {
+    if (e->cov_deferred && e->n_lanes > 1)
+        CU(cudaMemcpyAsync(&e->d_cov_carry[lane].nq, &nq, 4, cudaMemcpyHostToDevice, cov_stream(e)));
+    return 0;
+}
+
+extern "C" int bqc_cov_shard_boundary_lane(bqc_engine* e, int32_t lane, bqc_cov_shard* out) {
     memset(out, 0, sizeof(*out));
-    if (!e->cov_deferred && !e->cov_head_piece) { set_error(e, "bqc_cov_shard_boundary: engine is not in shard mode (bqc_cov_defer)"); return BQC_ERR_ARG; }
     uint32_t nq = 0;
-    int rc = cov_shard_sync(e, nq);
+    int rc = cov_shard_sync(e, "bqc_cov_shard_boundary", lane, nq);
     if (rc) return rc;
     if (e->cov_head_piece) {  // already resolved batch by batch: what matters to the pieces behind is the last record
         CovCarry c;
-        CU(cudaMemcpy(&c, e->d_cov_carry, sizeof(c), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(&c, e->d_cov_carry + lane, sizeof(c), cudaMemcpyDeviceToHost));
         out->n = c.first ? 0 : 1;   // (a count is not kept; non-zero = some record took part)
         out->last_rid = c.rid_prev;
         out->last_b = c.b_prev;
@@ -1778,7 +1855,7 @@ extern "C" int bqc_cov_shard_boundary(bqc_engine* e, bqc_cov_shard* out) {
     }
     out->n = nq;
     if (nq) {
-        const CovScratch& S = e->cov_scratch;
+        const CovScratch S = cov_lane_scratch(e, lane);
         CU(cudaMemcpy(&out->first_rid, S.q_rid, 4, cudaMemcpyDeviceToHost));
         CU(cudaMemcpy(&out->first_b, S.q_b, 4, cudaMemcpyDeviceToHost));
         CU(cudaMemcpy(&out->last_rid, S.q_rid + (nq - 1), 4, cudaMemcpyDeviceToHost));
@@ -1787,15 +1864,14 @@ extern "C" int bqc_cov_shard_boundary(bqc_engine* e, bqc_cov_shard* out) {
     return 0;
 }
 
-extern "C" int bqc_cov_shard_function(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint16_t* table1002) {
-    if (!e->cov_deferred && !e->cov_head_piece) { set_error(e, "bqc_cov_shard_function: engine is not in shard mode"); return BQC_ERR_ARG; }
+extern "C" int bqc_cov_shard_function_lane(bqc_engine* e, int32_t lane, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint16_t* table1002) {
     uint32_t nq = 0;
-    int rc = cov_shard_sync(e, nq);
+    int rc = cov_shard_sync(e, "bqc_cov_shard_function", lane, nq);
     if (rc) return rc;
     for (uint32_t s = 0; s < kCovStates; ++s) table1002[s] = (uint16_t)s;   // no record: the state passes through
     if (e->cov_head_piece) {  // the first piece ends in the state it carries
         CovCarry c;
-        CU(cudaMemcpy(&c, e->d_cov_carry, sizeof(c), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(&c, e->d_cov_carry + lane, sizeof(c), cudaMemcpyDeviceToHost));
         if (!c.first) for (uint32_t s = 0; s < kCovStates; ++s) table1002[s] = (uint16_t)cov_state_index(c.p_prev);
         return 0;
     }
@@ -1803,10 +1879,14 @@ extern "C" int bqc_cov_shard_function(bqc_engine* e, int32_t have_prev, int32_t 
     rc = ensure_cov_scratch(e, nq);
     if (rc) return rc;
     if (!e->d_cov_fn) CU(cudaMalloc(&e->d_cov_fn, 1024 * 2 + kCovD * 4));
+    const CovScratch S = cov_lane_scratch(e, lane);
+    CovCarry* carry = e->d_cov_carry + lane;
     const uint32_t nblk = (nq + kCovRB - 1) / kCovRB;
-    k_cov_set_state<<<1, 1, 0, cov_stream(e)>>>(e->d_cov_carry, have_prev ? 0u : 1u, prev_rid, prev_b, 0u);
-    k_cov_tables<<<nblk, kCovBlockThreads, kCovBlockSmem, cov_stream(e)>>>(e->cov_scratch, e->d_cov_carry);
-    k_cov_shard_function<<<1, 1024, 0, cov_stream(e)>>>(e->cov_scratch, e->d_cov_carry, e->d_cov_fn);
+    rc = cov_lane_set_nq(e, lane, nq);
+    if (rc) return rc;
+    k_cov_set_state<<<1, 1, 0, cov_stream(e)>>>(carry, have_prev ? 0u : 1u, prev_rid, prev_b, 0u);
+    k_cov_tables<<<nblk, kCovBlockThreads, kCovBlockSmem, cov_stream(e)>>>(S, carry);
+    k_cov_shard_function<<<1, 1024, 0, cov_stream(e)>>>(S, carry, e->d_cov_fn);
     e->launches += 3;
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(cov_stream(e)));
@@ -1814,21 +1894,22 @@ extern "C" int bqc_cov_shard_function(bqc_engine* e, int32_t have_prev, int32_t 
     return 0;
 }
 
-extern "C" int bqc_cov_shard_run(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint32_t p_in, bqc_cov_shard* out) {
-    if (!e->cov_deferred && !e->cov_head_piece) { set_error(e, "bqc_cov_shard_run: engine is not in shard mode"); return BQC_ERR_ARG; }
+extern "C" int bqc_cov_shard_run_lane(bqc_engine* e, int32_t lane, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint32_t p_in, bqc_cov_shard* out) {
     uint32_t nq = 0;
-    int rc = cov_shard_sync(e, nq);
+    int rc = cov_shard_sync(e, "bqc_cov_shard_run", lane, nq);
     if (rc) return rc;
     memset(out->head, 0, sizeof(out->head));
     memset(out->tail, 0, sizeof(out->tail));
     out->span = 0;
     out->n = nq;
+    CovCarry* carry = e->d_cov_carry + lane;
+    int32_t* cd = e->d_cov_d + (uint64_t)lane * 2 * kCovD;
     if (e->cov_head_piece) {  // nothing left to resolve: report the two windows that are still open
         CovCarry c;
-        CU(cudaMemcpy(&c, e->d_cov_carry, sizeof(c), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(&c, carry, sizeof(c), cudaMemcpyDeviceToHost));
         out->n = c.first ? 0 : 1;
         out->span = c.xc;
-        CU(cudaMemcpy(out->tail, e->d_cov_d + (uint64_t)c.parity * kCovD, sizeof(out->tail), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(out->tail, cd + (uint64_t)c.parity * kCovD, sizeof(out->tail), cudaMemcpyDeviceToHost));
         return 0;
     }
     if (!nq) return 0;
@@ -1836,28 +1917,39 @@ extern "C" int bqc_cov_shard_run(bqc_engine* e, int32_t have_prev, int32_t prev_
     if (rc) return rc;
     if (!e->d_cov_fn) CU(cudaMalloc(&e->d_cov_fn, 1024 * 2 + kCovD * 4));
     int32_t* d_head = (int32_t*)(e->d_cov_fn + 1024);
+    const CovScratch S = cov_lane_scratch(e, lane);
     BatchView B;
     memset(&B, 0, sizeof(B));
     CU(cudaMemsetAsync(e->d_cov_scratch, 0, e->cov_ctl_bytes, cov_stream(e)));
-    CU(cudaMemsetAsync(e->d_cov_d, 0, 2 * kCovD * 4, cov_stream(e)));
-    k_cov_set_state<<<1, 1, 0, cov_stream(e)>>>(e->d_cov_carry, have_prev ? 0u : 1u, prev_rid, prev_b, p_in);
+    CU(cudaMemsetAsync(cd, 0, 2 * kCovD * 4, cov_stream(e)));
+    rc = cov_lane_set_nq(e, lane, nq);
+    if (rc) return rc;
+    k_cov_set_state<<<1, 1, 0, cov_stream(e)>>>(carry, have_prev ? 0u : 1u, prev_rid, prev_b, p_in);
     {
         ProfScope prof(e, 3, cov_stream(e));
-        rc = launch_cov_resolve(e, 0, B, nq, false);
+        rc = launch_cov_resolve(e, (uint32_t)lane, S, B, nq, false);
         if (rc) return rc;
-        k_cov_head<<<1, 1024, 0, cov_stream(e)>>>(B, e->cov_scratch, e->d_cov_carry, d_head);
-        k_cov_carry<<<1, 1024, 0, cov_stream(e)>>>(B, e->cov_scratch, e->d_cov_carry, e->d_cov_d);
+        k_cov_head<<<1, 1024, 0, cov_stream(e)>>>(B, S, carry, d_head);
+        k_cov_carry<<<1, 1024, 0, cov_stream(e)>>>(B, S, carry, cd);
         e->launches += 3;
     }
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(cov_stream(e)));
     CovCarry c;
-    CU(cudaMemcpy(&c, e->d_cov_carry, sizeof(c), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&c, carry, sizeof(c), cudaMemcpyDeviceToHost));
     out->span = c.xc;
     CU(cudaMemcpy(out->head, d_head, sizeof(out->head), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(out->tail, e->d_cov_d + (uint64_t)c.parity * kCovD, sizeof(out->tail), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out->tail, cd + (uint64_t)c.parity * kCovD, sizeof(out->tail), cudaMemcpyDeviceToHost));
     e->have_results = false;
     return 0;
+}
+
+extern "C" int bqc_cov_shard_boundary(bqc_engine* e, bqc_cov_shard* out) { return bqc_cov_shard_boundary_lane(e, 0, out); }
+extern "C" int bqc_cov_shard_function(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint16_t* table1002) {
+    return bqc_cov_shard_function_lane(e, 0, have_prev, prev_rid, prev_b, table1002);
+}
+extern "C" int bqc_cov_shard_run(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint32_t p_in, bqc_cov_shard* out) {
+    return bqc_cov_shard_run_lane(e, 0, have_prev, prev_rid, prev_b, p_in, out);
 }
 
 extern "C" void bqc_cov_shards_combine(const bqc_cov_shard* shards, int32_t n_shards, int64_t delta[101]) {

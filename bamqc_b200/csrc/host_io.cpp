@@ -901,30 +901,35 @@ int finish_and_write(const Cli& c, std::vector<Piece>& pieces, const bqc_bam_hea
             return 1;
         }
     if (N > 1) {
-        // the coverage windows across the cuts (include/bamqc_b200.h: bqc_cov_shard_*), then everything is summed
-        std::vector<bqc_cov_shard> sh((size_t)N);
-        for (int k = 0; k < N; ++k)
-            if (bqc_cov_shard_boundary(pieces[k].eng, &sh[k])) return report_submit_error(pieces[k].eng, c);
-        std::vector<int> have_prev(N, 0);
-        std::vector<int32_t> prid(N, 0);
-        std::vector<uint32_t> pb(N, 0);
-        for (int k = 1; k < N; ++k) {
-            have_prev[k] = have_prev[k - 1]; prid[k] = prid[k - 1]; pb[k] = pb[k - 1];
-            if (sh[k - 1].n) { have_prev[k] = 1; prid[k] = sh[k - 1].last_rid; pb[k] = sh[k - 1].last_b; }
+        // the coverage windows across the cuts (include/bamqc_b200.h: bqc_cov_shard_*), one lane (read group) after the
+        // other: each lane's records are a stream of their own; then everything is summed
+        const int n_lanes = bqc_n_lanes(pieces[0].eng);
+        std::vector<std::vector<int64_t>> delta((size_t)n_lanes, std::vector<int64_t>(101));
+        for (int lane = 0; lane < n_lanes; ++lane) {
+            std::vector<bqc_cov_shard> sh((size_t)N);
+            for (int k = 0; k < N; ++k)
+                if (bqc_cov_shard_boundary_lane(pieces[k].eng, lane, &sh[k])) return report_submit_error(pieces[k].eng, c);
+            std::vector<int> have_prev(N, 0);
+            std::vector<int32_t> prid(N, 0);
+            std::vector<uint32_t> pb(N, 0);
+            for (int k = 1; k < N; ++k) {
+                have_prev[k] = have_prev[k - 1]; prid[k] = prid[k - 1]; pb[k] = pb[k - 1];
+                if (sh[k - 1].n) { have_prev[k] = 1; prid[k] = sh[k - 1].last_rid; pb[k] = sh[k - 1].last_b; }
+            }
+            std::vector<std::vector<uint16_t>> fn((size_t)N, std::vector<uint16_t>(1002));
+            for (int k = 0; k < N; ++k)
+                if (bqc_cov_shard_function_lane(pieces[k].eng, lane, have_prev[k], prid[k], pb[k], fn[k].data())) return report_submit_error(pieces[k].eng, c);
+            uint32_t p = 0;
+            for (int k = 0; k < N; ++k) {
+                if (bqc_cov_shard_run_lane(pieces[k].eng, lane, have_prev[k], prid[k], pb[k], p, &sh[k])) return report_submit_error(pieces[k].eng, c);
+                if (sh[k].n) p = bqc_cov_apply(fn[k].data(), p);
+            }
+            bqc_cov_shards_combine(sh.data(), N, delta[lane].data());
         }
-        std::vector<std::vector<uint16_t>> fn((size_t)N, std::vector<uint16_t>(1002));
-        for (int k = 0; k < N; ++k)
-            if (bqc_cov_shard_function(pieces[k].eng, have_prev[k], prid[k], pb[k], fn[k].data())) return report_submit_error(pieces[k].eng, c);
-        uint32_t p = 0;
-        for (int k = 0; k < N; ++k) {
-            if (bqc_cov_shard_run(pieces[k].eng, have_prev[k], prid[k], pb[k], p, &sh[k])) return report_submit_error(pieces[k].eng, c);
-            if (sh[k].n) p = bqc_cov_apply(fn[k].data(), p);
-        }
-        int64_t delta[101];
-        bqc_cov_shards_combine(sh.data(), N, delta);
         for (int k = 1; k < N; ++k)
             if (bqc_merge_from(pieces[0].eng, pieces[k].eng)) return report_submit_error(pieces[0].eng, c);
-        if (bqc_poscov_adjust(pieces[0].eng, 0, delta)) return report_submit_error(pieces[0].eng, c);
+        for (int lane = 0; lane < n_lanes; ++lane)
+            if (bqc_poscov_adjust(pieces[0].eng, lane, delta[lane].data())) return report_submit_error(pieces[0].eng, c);
     }
     auto t_stats = std::chrono::steady_clock::now();
     if (bqc_write_bamqc(pieces[0].eng, hdr.sample_id, c.out.c_str())) {
@@ -997,7 +1002,7 @@ int run_file(Cli& c, TimePoint t_start) {
         else { rec_beg = blocks.empty() ? 0 : blocks.back().bbeg + (blocks.back().cbeg - blocks.back().bbeg) + blocks.back().clen + 8; skip = 0; }
     }
     std::vector<int> devices = c.devices;
-    if (raw || !seekable || hdr.n_lanes != 1) devices.resize(1);   // pieces need BGZF block boundaries and device-side framing
+    if (raw || !seekable) devices.resize(1);   // pieces need BGZF block boundaries and device-side framing
     std::vector<uint64_t> cut(1, rec_beg);
     if (devices.size() > 1) {
         const uint64_t span = file_size - rec_beg;

@@ -59,7 +59,8 @@ struct CovScratch {  // sized for the largest batch; reused by every batch and l
     uint32_t* q_b;
     uint32_t* q_iv;
     uint32_t* q_rec;                 // batch index of the record (complex CIGARs are re-walked)
-    unsigned long long* base;        // virtual coordinate of the record's begin
+    uint8_t* q_lane;                 // several read groups: lane of the record (shard mode collects all lanes in one queue)
+    unsigned long long* base;       // virtual coordinate of the record's begin
     uint32_t* ab;                    // covered interval [a, b) relative to base: a | b << 11; complex: p | bit 31
     uint16_t* tables;                // [block][1024] state -> state (COV_TABLE blocks)
     uint4* desc;                     // [block] {type, a, b, -}
@@ -170,11 +171,14 @@ __device__ __forceinline__ void cov_walk_cigar(const uint8_t* p, F emit) {
 // not duplicate, rID in the -c set) and their (rid, begin, interval), compacted in file order.
 // ------------------------------------------------------------------------------------------------
 // append != 0 (shard mode): the records are added behind the carry->nq already collected instead of replacing them.
+// kTagged (shard mode, several read groups): every record of the batch whatever its lane, each tagged with its lane
+// in S.q_lane; the queue is grouped by lane once the run has ended (engine.cu cov_lane_split).
+template <bool kTagged>
 __global__ void __launch_bounds__(kCovPrepThreads, 2) k_cov_prep(EngineView E, BatchView B, uint32_t lane, CovScratch S, CovCarry* carry, uint32_t append) {
     __shared__ uint32_t ws[33];
     __shared__ uint32_t s_tile;
     __shared__ unsigned long long s_base;
-    const LaneRecords LR = lane_records(B, lane);
+    const LaneRecords LR = kTagged ? LaneRecords{B.n_records, nullptr} : lane_records(B, lane);
     const uint32_t ntile = (LR.n + kCovPrepTile - 1u) / kCovPrepTile;
     const uint32_t have = append ? carry->nq : 0u;   // only tile 0 uses it, and the last tile overwrites it after tile 0 has published
     for (;;) {
@@ -191,7 +195,7 @@ __global__ void __launch_bounds__(kCovPrepThreads, 2) k_cov_prep(EngineView E, B
             if (r0 + k >= LR.n) continue;
             const uint32_t r = LR[r0 + k];
             recno[k] = r;
-            if (!lane_match(B, r, lane)) continue;
+            if (!kTagged && !lane_match(B, r, lane)) continue;
             const uint32_t off = B.offsets[r], avail = B.offsets[r + 1] - off;
             if (avail < 36u) continue;
             const uint8_t* p = B.bytes + off;
@@ -225,6 +229,7 @@ __global__ void __launch_bounds__(kCovPrepThreads, 2) k_cov_prep(EngineView E, B
         for (uint32_t k = 0; k < kCovPrepPer; ++k)
             if (flags & (1u << k)) {
                 S.q_rid[o] = rid[k]; S.q_b[o] = b[k]; S.q_iv[o] = iv[k]; S.q_rec[o] = recno[k];
+                if (kTagged) S.q_lane[o] = B.rec_lane[recno[k]];
                 ++o;
             }
         __syncthreads();
@@ -735,6 +740,17 @@ __global__ void __launch_bounds__(1024) k_cov_head(BatchView B, CovScratch S, co
     }
     __syncthreads();
     for (uint32_t i = threadIdx.x; i < kCovD; i += blockDim.x) head[i] = dn[i];
+}
+
+// Several read groups: the collected records in the order of `index` (k_lane_partition over S.q_lane: lane by lane,
+// file order inside a lane), so that every lane's records are one contiguous segment of (rid, b, iv).
+__global__ void k_cov_lane_gather(CovScratch S, const uint32_t* __restrict__ index, uint32_t n, int32_t* rid, uint32_t* b, uint32_t* iv) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const uint32_t j = index[i];
+        rid[i] = S.q_rid[j];
+        b[i] = S.q_b[j];
+        iv[i] = S.q_iv[j];
+    }
 }
 
 __global__ void k_cov_set_state(CovCarry* carry, uint32_t first, int32_t rid_prev, uint32_t b_prev, uint32_t p_prev) {

@@ -83,29 +83,45 @@ def _combine(lib, shard_arrays):
     return delta
 
 
+def _resolve(engine, piece, exchange, lanes):
+    """The protocol for the lanes of one piece at once: each exchange carries one row per lane, so there are three
+    exchanges whatever the number of lanes.  `lanes`: the keyword arguments that select a lane in the engine's calls."""
+    b = [engine.cov_shard_boundary(**kw) for kw in lanes]
+    bounds = exchange(np.array([[x.n, x.first_rid, x.first_b, x.last_rid, x.last_b] for x in b], dtype=np.int64))
+    prev = []
+    for lane in range(len(lanes)):
+        have_prev, prid, pb = 0, 0, 0
+        for k in range(piece):
+            if int(bounds[k][lane][0]) > 0:
+                have_prev, prid, pb = 1, int(bounds[k][lane][3]), int(bounds[k][lane][4])
+        prev.append((have_prev, prid, pb))
+    tables = exchange(np.stack([engine.cov_shard_function(*prev[lane], **kw) for lane, kw in enumerate(lanes)]))
+    shards = []
+    for lane, kw in enumerate(lanes):
+        p = 0
+        for k in range(piece):
+            if int(bounds[k][lane][0]) > 0:
+                p = int(engine.lib.bqc_cov_apply(np.ascontiguousarray(tables[k][lane], dtype=np.uint16).ctypes.data, p))
+        shards.append(_shard_to_array(engine.cov_shard_run(*prev[lane], p, **kw)))
+    shards = exchange(np.stack(shards))
+    return [_combine(engine.lib, [s[lane] for s in shards]) for lane in range(len(lanes))]
+
+
 def resolve_coverage_shards(engine, piece, exchange):
     """Coverage statistic of piece number `piece` (stream order) of a record stream cut across engines in shard mode
     (Engine.cov_defer()); call it on every piece after Engine.finish().  Returns the correction to add to the SUM of
     the pieces' poscov tables (Engine.poscov_adjust on the merged result) -- identical on every piece."""
-    b = engine.cov_shard_boundary()
-    bounds = exchange(np.array([b.n, b.first_rid, b.first_b, b.last_rid, b.last_b], dtype=np.int64))
-    have_prev, prid, pb = 0, 0, 0
-    for k in range(piece):
-        if int(bounds[k][0]) > 0:
-            have_prev, prid, pb = 1, int(bounds[k][3]), int(bounds[k][4])
-    table = engine.cov_shard_function(have_prev, prid, pb)
-    tables = exchange(table)
-    p = 0
-    for k in range(piece):
-        if int(bounds[k][0]) > 0:
-            p = int(engine.lib.bqc_cov_apply(np.ascontiguousarray(tables[k], dtype=np.uint16).ctypes.data, p))
-    sh = engine.cov_shard_run(have_prev, prid, pb, p)
-    shards = exchange(_shard_to_array(sh))
-    return _combine(engine.lib, shards)
+    return _resolve(engine, piece, exchange, [{}])[0]
 
 
-def resolve_coverage_local(engines):
-    """The same protocol for engines that live in one process (pieces in list order)."""
+def resolve_coverage_shards_lanes(engine, piece, exchange, n_lanes):
+    """resolve_coverage_shards for an engine with `n_lanes` read groups: every lane's records are a stream of their own,
+    cut where the file is cut.  Returns one correction per lane (Engine.poscov_adjust(delta[lane], lane)), with the
+    same three exchanges as one lane."""
+    return _resolve(engine, piece, exchange, [dict(lane=lane) for lane in range(n_lanes)])
+
+
+def _resolve_local(engines, resolve):
     import threading
     n = len(engines)
     slots = {}
@@ -123,11 +139,21 @@ def resolve_coverage_local(engines):
             res = [slots[(key, j)] for j in range(n)]
             barrier.wait()
             return res
-        out[k] = resolve_coverage_shards(engines[k], k, exchange)
+        out[k] = resolve(engines[k], k, exchange)
     ths = [threading.Thread(target=run, args=(k,)) for k in range(n)]
     [t.start() for t in ths]
     [t.join() for t in ths]
     return out[0]
+
+
+def resolve_coverage_local(engines):
+    """The same protocol for engines that live in one process (pieces in list order)."""
+    return _resolve_local(engines, resolve_coverage_shards)
+
+
+def resolve_coverage_local_lanes(engines, n_lanes):
+    """resolve_coverage_shards_lanes for engines that live in one process: one correction per lane."""
+    return _resolve_local(engines, lambda e, k, x: resolve_coverage_shards_lanes(e, k, x, n_lanes))
 
 
 def torch_exchange(device=None, group=None):

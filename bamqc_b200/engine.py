@@ -207,19 +207,19 @@ class Engine:
         """1: a piece of a stream whose entry state is unknown; 2: the first piece of the stream; 0: stand-alone."""
         self._check(self.lib.bqc_cov_defer(self.handle, int(mode)))
 
-    def cov_shard_boundary(self):
+    def cov_shard_boundary(self, lane=0):
         sh = _lib.bqc_cov_shard()
-        self._check(self.lib.bqc_cov_shard_boundary(self.handle, ctypes.byref(sh)))
+        self._check(self.lib.bqc_cov_shard_boundary_lane(self.handle, int(lane), ctypes.byref(sh)))
         return sh
 
-    def cov_shard_function(self, have_prev, prev_rid, prev_b):
+    def cov_shard_function(self, have_prev, prev_rid, prev_b, lane=0):
         out = np.zeros(1002, dtype=np.uint16)
-        self._check(self.lib.bqc_cov_shard_function(self.handle, int(have_prev), int(prev_rid), int(prev_b), out.ctypes.data))
+        self._check(self.lib.bqc_cov_shard_function_lane(self.handle, int(lane), int(have_prev), int(prev_rid), int(prev_b), out.ctypes.data))
         return out
 
-    def cov_shard_run(self, have_prev, prev_rid, prev_b, p_in):
+    def cov_shard_run(self, have_prev, prev_rid, prev_b, p_in, lane=0):
         sh = _lib.bqc_cov_shard()
-        self._check(self.lib.bqc_cov_shard_run(self.handle, int(have_prev), int(prev_rid), int(prev_b), int(p_in), ctypes.byref(sh)))
+        self._check(self.lib.bqc_cov_shard_run_lane(self.handle, int(lane), int(have_prev), int(prev_rid), int(prev_b), int(p_in), ctypes.byref(sh)))
         return sh
 
     def poscov_adjust(self, delta, lane=0):

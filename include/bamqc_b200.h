@@ -174,7 +174,9 @@ int bqc_merge_from(bqc_engine* dst, bqc_engine* src);
  *   4. bqc_cov_shards_combine  (host arithmetic, any rank) -> what to add to the SUM of the pieces' poscov tables,
  *                                 including the end-of-run flush (src/bamqualcheck.cpp:447-453); apply it to the
  *                                 merged result with bqc_poscov_adjust.
- * Single read group only.  Pieces are numbered in stream order. */
+ * Pieces are numbered in stream order.  With several read groups every lane's records, in file order, are a stream of
+ * their own: run steps 1-4 once per lane with the *_lane calls and apply each lane's delta with
+ * bqc_poscov_adjust(e, lane, ...).  The calls without a lane are the lane 0 case. */
 typedef struct bqc_cov_shard {
     uint64_t n;                  /* records of the piece that take part in the statistic */
     int32_t first_rid, last_rid;
@@ -190,6 +192,9 @@ int bqc_cov_defer(bqc_engine* e, int on);   /* after bqc_reset, before the first
 int bqc_cov_shard_boundary(bqc_engine* e, bqc_cov_shard* out);
 int bqc_cov_shard_function(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint16_t* table1002);
 int bqc_cov_shard_run(bqc_engine* e, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint32_t p_in, bqc_cov_shard* out);
+int bqc_cov_shard_boundary_lane(bqc_engine* e, int32_t lane, bqc_cov_shard* out);
+int bqc_cov_shard_function_lane(bqc_engine* e, int32_t lane, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint16_t* table1002);
+int bqc_cov_shard_run_lane(bqc_engine* e, int32_t lane, int32_t have_prev, int32_t prev_rid, uint32_t prev_b, uint32_t p_in, bqc_cov_shard* out);
 void bqc_cov_shards_combine(const bqc_cov_shard* shards, int32_t n_shards, int64_t delta[101]);
 int bqc_poscov_adjust(bqc_engine* e, int32_t lane, const int64_t delta[101]);
 /* State after a piece whose function is `table1002`, entered in state p (0..1000 or 2000). */
