@@ -5,5 +5,5 @@ The product is the CUDA/C++ shared library ``libbamqc_b200.so`` (C ABI in ``incl
 ABI used by the tests, ``bench.py`` and the multi-GPU (torch.distributed / NCCL) merge.
 """
 from ._lib import load_library, library_path, build  # noqa: F401
-from .engine import Engine, Batch, BamQCError, FIELDS  # noqa: F401
+from .engine import Engine, Batch, BamQCError, FIELDS, parse_sam_header  # noqa: F401
 from . import synth  # noqa: F401

@@ -90,6 +90,10 @@ PROTOTYPES = {
     "bqc_stream_unknown_start": (ctypes.c_int, [_vp]),
     "bqc_stream_skipped": (ctypes.c_int, [_vp, _P(_u64)]),
     "bqc_frames_repaired": (_u64, [_vp]),
+    "bqc_set_ref_names": (ctypes.c_int, [_vp, _i32, _P(ctypes.c_char_p)]),
+    "bqc_submit_sam": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, ctypes.c_int]),
+    "bqc_sam_to_bam": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, _vp, _u64, _P(_u64), _P(_u64)]),
+    "bqc_sam_host_lines": (_u64, [_vp]),
     "bqc_records_seen": (_u64, [_vp]),
     "bqc_batch_prepare": (ctypes.c_int, [_vp, _vp, ctypes.c_size_t, _vp, _u64, _P(_vp)]),
     "bqc_batch_run": (ctypes.c_int, [_vp, _vp]),
@@ -132,6 +136,7 @@ PROTOTYPES = {
     "bqc_write_bamqc": (ctypes.c_int, [_vp, ctypes.c_char_p, ctypes.c_char_p]),
     "bqc_parse_bam_header": (ctypes.c_size_t, [_vp, ctypes.c_size_t, _P(bqc_bam_header)]),
     "bqc_free_bam_header": (None, [_P(bqc_bam_header)]),
+    "bqc_parse_sam_header": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_size_t, _P(bqc_bam_header), _P(ctypes.c_size_t)]),
     "bqc_frame_records": (_u64, [_vp, ctypes.c_size_t, _vp, _u64]),
     "bqc_frame_records_mt": (_u64, [_vp, ctypes.c_size_t, _vp, _u64, _i32, _i32]),
     "bqc_bgzf_inflate": (_u64, [_vp, _u64, _vp, _u64, _i32]),
@@ -150,6 +155,7 @@ SYNTH_PROTOTYPES = {
     "bqc_synth_records": (ctypes.c_int, [_P(bqc_synth_params), _vp, _u64, _P(_u64), _vp, _u64, _P(_u64)]),
     "bqc_synth_write_bam": (ctypes.c_int, [ctypes.c_char_p, _P(bqc_synth_params), ctypes.c_char_p, _vp, _u64, ctypes.c_int]),
     "bqc_synth_bgzf_compress": (_u64, [_vp, _u64, ctypes.c_int, _vp, _u64]),
+    "bqc_synth_write_sam": (ctypes.c_int, [ctypes.c_char_p, _P(bqc_synth_params), ctypes.c_char_p, _vp, _u64]),
 }
 
 

@@ -30,6 +30,8 @@
 #include "kernels.cuh"
 #include "kernel_frame.cuh"
 #include "kernel_inflate.cuh"
+#include "kernel_sam.cuh"
+#include "sam_text.h"
 
 using namespace bqc;
 
@@ -140,6 +142,13 @@ struct Slot {  // one half of the staging double buffer
     InflateBlock* h_blocks = nullptr;  // pinned
     InflateBlock* d_blocks = nullptr;
     uint32_t* d_ictl = nullptr;        // ticket, error
+    // SAM text (kernel_sam.cuh), allocated on the first SAM submission: the text, its line ends, the packed per-line
+    // sizes and their tile sums, and a batch with room for the encoded records (up to twice the text)
+    uint8_t* d_text = nullptr;
+    uint32_t* d_lend = nullptr;
+    unsigned long long *d_sz = nullptr, *d_sbsum = nullptr;
+    SamCtl* d_sctl = nullptr;
+    DeviceBatch sam;
 };
 
 struct bqc_engine {
@@ -204,8 +213,9 @@ struct bqc_engine {
     struct Task {
         int slot; const uint8_t* h2d_src; size_t span; uint64_t n_records; uint32_t max_lseq;
         int mode;          // 0: framed by the host (offsets + meta in the slot), 1: raw stream bytes, framed on the device,
-                           // 2: BGZF blocks, inflated and framed on the device
-        uint32_t n_blocks = 0, inflated = 0, skip = 0;  // mode 2: BGZF blocks, their total inflated size, leading non-record bytes
+                           // 2: BGZF blocks, inflated and framed on the device, 3: SAM text, encoded on the device
+        uint32_t n_blocks = 0, inflated = 0, skip = 0;  // mode 2: BGZF blocks, their total inflated size, leading non-record bytes;
+                                                        // mode 3: skip = 1 when the last line has no newline
         bool seek = false;  // the stream starts inside a record: find the first record boundary (k_frame_seek)
         bool must_align;   // the bytes must end on a record boundary (whole-record submissions, last stream chunk)
     };
@@ -259,6 +269,15 @@ struct bqc_engine {
     double prof_ms[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     uint64_t prof_n[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
     uint64_t blocks_per_slot = 0;  // capacity of the BGZF block table of a slot
+    // SAM text: the @SQ names (bqc_set_ref_names) as the host encoder's map and as the device's sorted table
+    bool have_sam_refs = false;
+    std::map<std::string, int32_t> sam_ref_id;
+    char* d_sam_blob = nullptr;
+    uint32_t* d_sam_off = nullptr;
+    int32_t* d_sam_id = nullptr;
+    SamRefs sam_refs = {nullptr, nullptr, nullptr, 0};
+    uint64_t sam_line_cap = 0, sam_rec_cap = 0, sam_byte_cap = 0;   // per slot
+    std::atomic<uint64_t> sam_host_lines{0};
     int inflate_bps = 0;
 
     // results (after finish)
@@ -355,6 +374,8 @@ extern "C" void bqc_destroy(bqc_engine* e) {
         cudaFree(s.d_cin); cudaFree(s.d_blocks); cudaFree(s.d_ictl);
         cudaFree(s.d_frame); cudaFree(s.d_ws); cudaFree(s.d_we); cudaFree(s.d_wc); cudaFree(s.d_ws2); cudaFree(s.d_we2); cudaFree(s.d_wc2); cudaFree(s.d_bsum); cudaFree(s.d_bbase);
         free_device_batch(s.dev);
+        cudaFree(s.d_text); cudaFree(s.d_lend); cudaFree(s.d_sz); cudaFree(s.d_sbsum); cudaFree(s.d_sctl);
+        free_device_batch(s.sam);
         if (s.done) cudaEventDestroy(s.done);
         if (s.framed) cudaEventDestroy(s.framed);
         if (s.inflated) cudaEventDestroy(s.inflated);
@@ -376,6 +397,7 @@ extern "C" void bqc_destroy(bqc_engine* e) {
     cudaFree(e->d_hash);
     cudaFree(e->d_lane_names);
     cudaFree(e->d_lane_off);
+    cudaFree(e->d_sam_blob); cudaFree(e->d_sam_off); cudaFree(e->d_sam_id);
     if (e->copied) cudaEventDestroy(e->copied);
     if (e->cov_done) cudaEventDestroy(e->cov_done);
     if (e->cov_go) cudaEventDestroy(e->cov_go);
@@ -482,6 +504,9 @@ extern "C" int bqc_create(const bqc_config* cfg, bqc_engine** out) {
     if (e->staging_bytes > 0xF0000000ull) e->staging_bytes = 0xF0000000ull;
     e->max_records_per_slot = e->staging_bytes / 36 + 16;  // a record is at least 37 bytes (block_size + 32 fixed + a NUL name)
     e->blocks_per_slot = e->staging_bytes / 4096 + 4096;   // BGZF blocks per submission (larger inputs are split)
+    e->sam_line_cap = e->staging_bytes / kSamMinLine + 16;   // a fast SAM line is at least 22 bytes; more lines fall back
+    e->sam_rec_cap = e->sam_line_cap;
+    e->sam_byte_cap = std::min<uint64_t>(2 * e->staging_bytes, 0xF0000000ull);   // a fast line encodes to at most twice its text
     if (const char* v = getenv("BQC_STATS_BPS")) e->tune_stats_bps = atoi(v);
     if (const char* v = getenv("BQC_STATS_STAGE")) e->tune_stats_stage = atoi(v);
     if (const char* v = getenv("BQC_COV_BPS")) e->tune_cov_bps = std::max(1, std::min(6, atoi(v)));
@@ -1204,7 +1229,10 @@ static int commit_task(bqc_engine* e, const bqc_engine::Task& t) {
 }
 
 // stream task, stage A: carry the partial record of the previous buffer, copy the new bytes, frame on the device
+static int sam_stage_a(bqc_engine* e, const bqc_engine::Task& t);
+static int sam_stage_b(bqc_engine* e, const bqc_engine::Task& t);
 static int stream_stage_a(bqc_engine* e, const bqc_engine::Task& t) {
+    if (t.mode == 3) return sam_stage_a(e, t);
     Slot& s = e->slots[t.slot];
     DeviceBatch& d = s.dev;
     const Slot* prev = e->last_stream_slot >= 0 ? &e->slots[e->last_stream_slot] : nullptr;
@@ -1263,6 +1291,7 @@ static int stream_stage_a(bqc_engine* e, const bqc_engine::Task& t) {
 
 // stage B: read the frame header back (record count, longest read), launch the coverage and the table kernels
 static int stream_stage_b(bqc_engine* e, const bqc_engine::Task& t) {
+    if (t.mode == 3) return sam_stage_b(e, t);
     Slot& s = e->slots[t.slot];
     DeviceBatch& d = s.dev;
     auto t_b0 = std::chrono::steady_clock::now();
@@ -1630,6 +1659,235 @@ extern "C" uint64_t bqc_frames_repaired(bqc_engine* e) { drain_commits(e); retur
 extern "C" uint64_t bqc_records_seen(bqc_engine* e) { drain_commits(e); return e->records_seen; }
 
 // ------------------------------------------------------------------------------------------------
+// SAM text (kernel_sam.cuh): whole lines in, BAM records out on the device; a submission with a line outside the
+// fast grammar (sam_parse.h) is encoded on the host with sam_line_to_bam and run as host-framed batches
+// ------------------------------------------------------------------------------------------------
+static int ensure_sam_slot(bqc_engine* e, Slot& s) {
+    if (s.d_text) return 0;
+    CU(cudaSetDevice(e->cfg.device));
+    CU(cudaMalloc(&s.d_text, e->staging_bytes + 512));
+    CU(cudaMemset(s.d_text, 0, e->staging_bytes + 512));
+    CU(cudaMalloc(&s.d_lend, (e->sam_line_cap + 1) * 4));
+    CU(cudaMalloc(&s.d_sz, (e->sam_line_cap + 1) * 8));
+    const uint64_t tiles = e->sam_line_cap / (kSamScanThreads * kSamScanPer) + 2;
+    const uint64_t nl_blocks = (e->staging_bytes + 1) / (kSamNlThreads * kSamNlPer) + 2;
+    CU(cudaMalloc(&s.d_sbsum, std::max(tiles, nl_blocks) * 8));
+    CU(cudaMalloc(&s.d_sctl, sizeof(SamCtl)));
+    return alloc_device_batch(e, s.sam, e->sam_byte_cap, e->sam_rec_cap);
+}
+
+// stage A: text over PCIe, line ends, sizes, scan, records; the frame header goes back to the host
+static int sam_stage_a(bqc_engine* e, const bqc_engine::Task& t) {
+    Slot& s = e->slots[t.slot];
+    DeviceBatch& d = s.sam;
+    CU(cudaMemcpyAsync(s.d_text, t.h2d_src, t.span, cudaMemcpyHostToDevice, e->copy));
+    CU(cudaEventRecord(e->copied, e->copy));
+    CU(cudaStreamWaitEvent(e->frames, e->copied, 0));
+    const uint32_t n = (uint32_t)t.span + t.skip;
+    {
+        ProfScope prof(e, 10, e->frames);
+        if (t.skip) CU(cudaMemsetAsync(s.d_text + t.span, '\n', 1, e->frames));
+        CU(cudaMemsetAsync(s.d_sctl, 0, sizeof(SamCtl), e->frames));
+        const uint32_t nl_blocks = (uint32_t)((n + kSamNlThreads * kSamNlPer - 1) / (kSamNlThreads * kSamNlPer));
+        k_sam_nl_count<<<nl_blocks, kSamNlThreads, 0, e->frames>>>(s.d_text, n, s.d_sbsum);
+        k_sam_scan_top<<<1, 1024, 0, e->frames>>>(s.d_sbsum, nl_blocks, nullptr, 1, 0, &s.d_sctl->lines);
+        k_sam_nl_emit<<<nl_blocks, kSamNlThreads, 0, e->frames>>>(s.d_text, n, s.d_sbsum, s.d_lend, e->sam_line_cap);
+        // lines of 300-700 bytes: a few per thread already fill the GPU; the grid-stride loop takes the rest
+        const uint64_t est = std::min<uint64_t>(e->sam_line_cap, n / 200 + 1);
+        const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((est + kSamLineThreads - 1) / kSamLineThreads, (uint64_t)e->n_sm * 16));
+        k_sam_size<<<grid, kSamLineThreads, 0, e->frames>>>(s.d_text, s.d_lend, s.d_sctl, e->sam_line_cap, e->sam_refs, s.d_sz);
+        const uint32_t tiles = (uint32_t)(std::min<uint64_t>(e->sam_line_cap, n) / (kSamScanThreads * kSamScanPer) + 1);
+        k_sam_scan_tiles<<<tiles, kSamScanThreads, 0, e->frames>>>(s.d_sz, &s.d_sctl->lines, e->sam_line_cap, s.d_sbsum);
+        k_sam_scan_top<<<1, 1024, 0, e->frames>>>(s.d_sbsum, 0, &s.d_sctl->lines, kSamScanThreads * kSamScanPer, e->sam_line_cap, &s.d_sctl->packed);
+        k_sam_scan_apply<<<tiles, kSamScanThreads, 0, e->frames>>>(s.d_sz, &s.d_sctl->lines, e->sam_line_cap, s.d_sbsum);
+        k_sam_encode<<<grid, kSamLineThreads, 0, e->frames>>>(s.d_text, s.d_lend, s.d_sctl, e->sam_line_cap, e->sam_rec_cap, e->sam_byte_cap, e->sam_refs, s.d_sz,
+                                                                d.bytes, d.offsets, s.d_frame);
+        e->launches += 8;
+    }
+    if (e->n_lanes > 1) {  // several read groups: as for a device-framed stream
+        k_frame_lanes<<<e->n_sm * 4, 256, 0, e->frames>>>(d.bytes, s.d_frame, d.offsets, e->d_lane_names, e->d_lane_off, e->n_lanes, d.rec_lane);
+        e->launches += 1;
+        int rcp = launch_lane_partition(e, d, &s.d_frame->n_records, 0, e->frames);
+        if (rcp) return rcp;
+    }
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(s.h_frame, s.d_frame, sizeof(FrameResult), cudaMemcpyDeviceToHost, e->frames));
+    CU(cudaEventRecord(s.framed, e->frames));
+    return 0;
+}
+
+// The host encoder over every line of text[0..n): records into enc, their starts (and the end) into offs.  Returns
+// false at the first line sam_line_to_bam rejects (enc/offs then hold the records in front of it).
+static bool sam_host_encode(bqc_engine* e, const uint8_t* text, size_t n, std::vector<uint8_t>& enc, std::vector<uint64_t>& offs) {
+    enc.clear();
+    offs.assign(1, 0);
+    std::string line;
+    uint64_t lines = 0;
+    bool ok = true;
+    for (size_t p = 0; p < n;) {
+        const uint8_t* q = (const uint8_t*)memchr(text + p, '\n', n - p);
+        const size_t end = q ? (size_t)(q - text) : n;
+        line.assign((const char*)text + p, end - p);
+        p = end + 1;
+        if (!line.empty() && line.back() == '\r') line.pop_back();
+        if (line.empty()) continue;
+        ++lines;
+        if (!sam_line_to_bam(line, e->sam_ref_id, enc)) { ok = false; break; }
+        offs.push_back(enc.size());
+    }
+    e->sam_host_lines += lines;
+    return ok;
+}
+
+static int sam_bad_line(bqc_engine* e) {
+    e->host_error.code = BQC_ERR_BAD_RECORD;
+    e->host_error.record = e->records_seen;
+    snprintf(e->host_error.message, sizeof(e->host_error.message), "ERROR: Could not read record from BAM File (malformed SAM line, record %llu)", (unsigned long long)e->records_seen);
+    set_error(e, "%s", e->host_error.message);
+    return BQC_ERR_BAD_RECORD;
+}
+
+// stage B: run the device's records, or encode the submission on the host and run it as host-framed batches
+static int sam_stage_b(bqc_engine* e, const bqc_engine::Task& t) {
+    Slot& s = e->slots[t.slot];
+    CU(cudaEventSynchronize(s.framed));
+    const FrameResult fr = *s.h_frame;
+    if (!fr.bad) {
+        DeviceBatch& d = s.sam;
+        d.max_lseq = fr.max_lseq;
+        d.n_records = fr.n_records;
+        d.n_bytes = fr.end;
+        d.first_record = e->records_seen;
+        d.base = d.bytes;
+        e->records_seen += fr.n_records;
+        if (fr.n_records) {
+            CU(cudaStreamWaitEvent(e->compute, s.framed, 0));
+            int rc = run_device_batch(e, d);
+            if (rc) return rc;
+        }
+        CU(cudaEventRecord(s.done, e->compute));
+        return 0;
+    }
+    std::vector<uint8_t> enc;
+    std::vector<uint64_t> offs;
+    const bool ok = sam_host_encode(e, t.h2d_src, t.span, enc, offs);
+    const uint64_t n = offs.size() - 1;
+    for (uint64_t r0 = 0; r0 < n;) {   // batches that fit the slot's host-framed capacities, one after the other
+        uint64_t r1 = r0 + 1;
+        while (r1 < n && r1 - r0 < e->max_records_per_slot && offs[r1 + 1] - offs[r0] <= e->staging_bytes) ++r1;
+        if (offs[r1] - offs[r0] > e->staging_bytes) { set_error(e, "bqc_submit_sam: a record is larger than the staging buffer"); return BQC_ERR_ARG; }
+        bqc_engine::Task b = t;
+        b.mode = 0;
+        b.n_records = r1 - r0;
+        b.span = (size_t)(offs[r1] - offs[r0]);
+        b.h2d_src = enc.data() + offs[r0];
+        host_scan_pass1(e, enc.data(), offs.data() + r0, b.n_records, s.h_offsets, e->n_lanes > 1 ? s.h_lane : nullptr, b.max_lseq);
+        int rc = commit_task(e, b);
+        if (rc) return rc;
+        CU(cudaEventSynchronize(s.done));   // the slot's buffers are reused by the next batch
+        r0 = r1;
+    }
+    if (!ok) return sam_bad_line(e);
+    CU(cudaEventRecord(s.done, e->compute));
+    return 0;
+}
+
+extern "C" int bqc_set_ref_names(bqc_engine* e, int32_t n, const char* const* names) {
+    if (n != e->cfg.n_ref || (n > 0 && !names)) { set_error(e, "bqc_set_ref_names: %d names for an engine of %d references", n, e->cfg.n_ref); return BQC_ERR_ARG; }
+    CU(cudaSetDevice(e->cfg.device));
+    { int arc = drain_commits(e); if (arc) return arc; }
+    for (auto& sl : e->slots) { int rc = wait_slot(e, sl); if (rc) return rc; }
+    std::vector<std::string> v(names, names + n);
+    std::string blob;
+    std::vector<uint32_t> off;
+    std::vector<int32_t> id;
+    sam_refs_build(v, blob, off, id);
+    e->sam_ref_id.clear();
+    for (int32_t i = 0; i < n; ++i) e->sam_ref_id.insert({v[i], i});   // first of duplicate names wins
+    cudaFree(e->d_sam_blob); cudaFree(e->d_sam_off); cudaFree(e->d_sam_id);
+    e->d_sam_blob = nullptr; e->d_sam_off = nullptr; e->d_sam_id = nullptr;
+    CU(cudaMalloc(&e->d_sam_blob, blob.size() + 1));
+    CU(cudaMalloc(&e->d_sam_off, off.size() * 4));
+    CU(cudaMalloc(&e->d_sam_id, id.size() * 4 + 4));
+    CU(cudaMemcpy(e->d_sam_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(e->d_sam_off, off.data(), off.size() * 4, cudaMemcpyHostToDevice));
+    if (!id.empty()) CU(cudaMemcpy(e->d_sam_id, id.data(), id.size() * 4, cudaMemcpyHostToDevice));
+    e->sam_refs = {e->d_sam_blob, e->d_sam_off, e->d_sam_id, (int32_t)id.size()};
+    e->have_sam_refs = true;
+    return 0;
+}
+
+static int sam_check(bqc_engine* e, const char* fn, const uint8_t* text, size_t n, bool last) {
+    if (e->finished) { set_error(e, "%s after bqc_finish (call bqc_reset)", fn); return BQC_ERR_ARG; }
+    if (!e->have_sam_refs) { set_error(e, "%s: call bqc_set_ref_names first", fn); return BQC_ERR_ARG; }
+    if (n > e->staging_bytes) { set_error(e, "%s: %zu bytes exceed the staging capacity %llu", fn, n, (unsigned long long)e->staging_bytes); return BQC_ERR_ARG; }
+    if (n && !last && text[n - 1] != '\n') { set_error(e, "%s: the text does not end at a line end", fn); return BQC_ERR_ARG; }
+    return 0;
+}
+
+extern "C" int bqc_submit_sam(bqc_engine* e, const void* text, size_t n, int last) {
+    const uint8_t* src = (const uint8_t*)text;
+    int rc = sam_check(e, "bqc_submit_sam", src, n, last != 0);
+    if (rc) return rc;
+    if (e->async_rc) return e->async_rc;
+    if (n == 0) return 0;
+    CU(cudaSetDevice(e->cfg.device));
+    Slot& s = e->slots[e->next_slot];
+    if ((rc = ensure_slot(e, s)) || (rc = ensure_sam_slot(e, s)) || (rc = wait_slot(e, s))) return rc;
+    bqc_engine::Task t;
+    t.slot = e->next_slot;
+    t.n_records = 0;
+    t.max_lseq = 0;
+    t.mode = 3;
+    t.must_align = true;
+    t.span = n;
+    t.skip = src[n - 1] != '\n' ? 1u : 0u;
+    t.h2d_src = h2d_source(e, s, src, n);
+    enqueue_task(e, s, t);
+    return 0;
+}
+
+extern "C" int bqc_sam_to_bam(bqc_engine* e, const void* text, size_t n, uint8_t* out, uint64_t cap, uint64_t* n_bytes, uint64_t* n_records) {
+    const uint8_t* src = (const uint8_t*)text;
+    *n_bytes = 0;
+    *n_records = 0;
+    int rc = sam_check(e, "bqc_sam_to_bam", src, n, true);
+    if (rc) return rc;
+    if (n == 0) return 0;
+    CU(cudaSetDevice(e->cfg.device));
+    { int arc = drain_commits(e); if (arc) return arc; }
+    Slot& s = e->slots[e->next_slot];
+    if ((rc = ensure_slot(e, s)) || (rc = ensure_sam_slot(e, s)) || (rc = wait_slot(e, s))) return rc;
+    bqc_engine::Task t;
+    t.slot = e->next_slot;
+    t.mode = 3;
+    t.span = n;
+    t.skip = src[n - 1] != '\n' ? 1u : 0u;
+    t.h2d_src = h2d_source(e, s, src, n);
+    if ((rc = sam_stage_a(e, t))) return rc;
+    CU(cudaEventSynchronize(s.framed));
+    const FrameResult fr = *s.h_frame;
+    if (!fr.bad) {
+        if (fr.end > cap) { set_error(e, "bqc_sam_to_bam: %u record bytes exceed the output capacity", fr.end); return BQC_ERR_ARG; }
+        CU(cudaMemcpy(out, s.sam.bytes, fr.end, cudaMemcpyDeviceToHost));
+        *n_bytes = fr.end;
+        *n_records = fr.n_records;
+        return 0;
+    }
+    std::vector<uint8_t> enc;
+    std::vector<uint64_t> offs;
+    const bool ok = sam_host_encode(e, t.h2d_src, t.span, enc, offs);
+    if (offs.back() > cap) { set_error(e, "bqc_sam_to_bam: %llu record bytes exceed the output capacity", (unsigned long long)offs.back()); return BQC_ERR_ARG; }
+    memcpy(out, enc.data(), (size_t)offs.back());
+    *n_bytes = offs.back();
+    *n_records = offs.size() - 1;
+    if (!ok) { set_error(e, "bqc_sam_to_bam: SAM line of record %llu is malformed", (unsigned long long)*n_records); return BQC_ERR_BAD_RECORD; }
+    return 0;
+}
+
+extern "C" uint64_t bqc_sam_host_lines(bqc_engine* e) { drain_commits(e); return e->sam_host_lines; }
+
+// ------------------------------------------------------------------------------------------------
 // resident path
 // ------------------------------------------------------------------------------------------------
 extern "C" int bqc_batch_prepare(bqc_engine* e, const void* data, size_t n_bytes, const uint64_t* record_offsets, uint64_t n_records, bqc_batch** out) {
@@ -1703,10 +1961,14 @@ static const char* reference_message(int code) {
 
 extern "C" int bqc_get_error(bqc_engine* e, bqc_error_info* out) {
     memset(out, 0, sizeof(*out));
-    if (e->host_error.code) { *out = e->host_error; return 0; }
-    CU(cudaSetDevice(e->cfg.device));
     unsigned long long key = ~0ull;
-    CU(cudaMemcpy(&key, e->d_error, 8, cudaMemcpyDeviceToHost));
+    if (cudaSetDevice(e->cfg.device) != cudaSuccess || cudaMemcpy(&key, e->d_error, 8, cudaMemcpyDeviceToHost) != cudaSuccess) {
+        cudaGetLastError();
+        if (!e->host_error.code) { set_error(e, "bqc_get_error: reading the device error word failed"); return BQC_ERR_CUDA; }
+        key = ~0ull;
+    }
+    // the first offending record in file order wins, whether the host or the device found it
+    if (e->host_error.code && (key == ~0ull || ((unsigned long long)e->host_error.record << 8 | (uint32_t)e->host_error.code) <= key)) { *out = e->host_error; return 0; }
     if (key != ~0ull) {
         out->code = (int32_t)(key & 255);
         out->record = key >> 8;
@@ -1717,7 +1979,13 @@ extern "C" int bqc_get_error(bqc_engine* e, bqc_error_info* out) {
 
 extern "C" int bqc_sync(bqc_engine* e) {
     CU(cudaSetDevice(e->cfg.device));
-    { int arc = drain_commits(e); if (arc) return arc; }
+    const int arc = drain_commits(e);
+    if (arc) {   // the work enqueued in front of the failure still runs: its errors are final once it has
+        cudaStreamSynchronize(e->copy);
+        cudaStreamSynchronize(e->covs);
+        cudaStreamSynchronize(e->compute);
+        return arc;
+    }
     CU(cudaStreamSynchronize(e->copy));
     CU(cudaStreamSynchronize(e->covs));
     CU(cudaStreamSynchronize(e->compute));

@@ -10,6 +10,7 @@
 #include <zlib.h>
 
 #include <algorithm>
+#include <cerrno>
 #include <atomic>
 #include <chrono>
 #include <cstdint>
@@ -27,6 +28,7 @@
 #include <vector>
 
 #include "../../include/bamqc_b200.h"
+#include "sam_text.h"
 
 // ------------------------------------------------------------------------------------------------
 // BAM header
@@ -112,6 +114,24 @@ extern "C" void bqc_free_bam_header(bqc_bam_header* h) {
     free(h->lane_ids);
     free(h->sample_id);
     memset(h, 0, sizeof(*h));
+}
+
+// SAM header lines ('@' at the start; a trailing '\r' dropped) -> the binary BAM header -> the same parser
+extern "C" int bqc_parse_sam_header(const char* text, size_t n, bqc_bam_header* out, size_t* consumed) {
+    std::string head;
+    size_t p = 0;
+    while (p < n && text[p] == '@') {
+        const char* q = (const char*)memchr(text + p, '\n', n - p);
+        const size_t end = q ? (size_t)(q - text) : n;
+        size_t len = end - p;
+        if (len && text[p + len - 1] == '\r') --len;
+        head.append(text + p, len);
+        head += '\n';
+        p = q ? end + 1 : n;
+    }
+    *consumed = p;
+    const std::vector<uint8_t> bam = sam_header_to_bam(head);
+    return bqc_parse_bam_header(bam.data(), bam.size(), out) ? 0 : BQC_ERR_ARG;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -495,160 +515,6 @@ struct Cli {
     uint64_t staging_mb = 0;
     bool timing = false;
 };
-}  // namespace
-
-// ------------------------------------------------------------------------------------------------
-// SAM text on stdin (`bamqualcheck ... -`: src/bamqualcheck.cpp:252-260, src/CommandLineParser.hpp:88-107).  The
-// text is turned into the BAM records the engine consumes (SAM/BAM specification sections 1.4 and 4.2); the header
-// lines become a BAM header so that the one header parser serves both formats.
-// ------------------------------------------------------------------------------------------------
-namespace {
-template <typename T> void put_le(std::vector<uint8_t>& v, T x) { uint8_t b[sizeof(T)]; memcpy(b, &x, sizeof(T)); v.insert(v.end(), b, b + sizeof(T)); }
-
-std::vector<std::string> split_tabs(const std::string& line) {
-    std::vector<std::string> out;
-    size_t p = 0;
-    for (;;) {
-        size_t q = line.find('\t', p);
-        out.push_back(line.substr(p, q == std::string::npos ? std::string::npos : q - p));
-        if (q == std::string::npos) break;
-        p = q + 1;
-    }
-    return out;
-}
-
-// binary BAM header (magic, text, reference list) from SAM header lines
-std::vector<uint8_t> sam_header_to_bam(const std::string& text) {
-    std::vector<uint8_t> h = {'B', 'A', 'M', 1};
-    put_le<int32_t>(h, (int32_t)text.size());
-    h.insert(h.end(), text.begin(), text.end());
-    std::vector<std::pair<std::string, int32_t>> refs;
-    std::istringstream is(text);
-    std::string line;
-    while (std::getline(is, line)) {
-        if (line.compare(0, 3, "@SQ") != 0) continue;
-        std::string name;
-        int64_t len = 0;
-        for (const std::string& f : split_tabs(line)) {
-            if (f.compare(0, 3, "SN:") == 0) name = f.substr(3);
-            else if (f.compare(0, 3, "LN:") == 0) len = atoll(f.c_str() + 3);
-        }
-        refs.push_back({name, (int32_t)len});
-    }
-    put_le<int32_t>(h, (int32_t)refs.size());
-    for (auto& r : refs) {
-        put_le<int32_t>(h, (int32_t)r.first.size() + 1);
-        h.insert(h.end(), r.first.begin(), r.first.end());
-        h.push_back(0);
-        put_le<int32_t>(h, r.second);
-    }
-    return h;
-}
-
-// one SAM alignment line -> one BAM record appended to out (block_size prefix included); false if malformed
-bool sam_line_to_bam(const std::string& line, const std::map<std::string, int32_t>& ref_id, std::vector<uint8_t>& out) {
-    const std::vector<std::string> f = split_tabs(line);
-    if (f.size() < 11) return false;
-    auto rid_of = [&](const std::string& name, int32_t same) -> int32_t {
-        if (name == "*") return -1;
-        if (name == "=") return same;
-        auto it = ref_id.find(name);
-        return it == ref_id.end() ? -1 : it->second;
-    };
-    const int32_t rid = rid_of(f[2], -1), pos = (int32_t)atoll(f[3].c_str()) - 1;
-    const int32_t nrid = rid_of(f[6], rid), npos = (int32_t)atoll(f[7].c_str()) - 1, tlen = (int32_t)atoll(f[8].c_str());
-    const uint32_t flag = (uint32_t)atoi(f[1].c_str()), mapq = (uint32_t)atoi(f[4].c_str());
-    std::vector<uint32_t> cigar;
-    if (f[5] != "*") {
-        static const char ops[] = "MIDNSHP=X";
-        uint64_t n = 0;
-        bool have = false;
-        for (char ch : f[5]) {
-            if (ch >= '0' && ch <= '9') { n = n * 10 + (uint64_t)(ch - '0'); have = true; continue; }
-            const char* o = strchr(ops, ch);
-            if (!o || !have) return false;
-            cigar.push_back((uint32_t)(n << 4) | (uint32_t)(o - ops));
-            n = 0;
-            have = false;
-        }
-        if (have) return false;
-    }
-    const std::string seq = f[9] == "*" ? std::string() : f[9];
-    const size_t start = out.size();
-    put_le<int32_t>(out, 0);  // block_size, patched below
-    put_le<int32_t>(out, rid);
-    put_le<int32_t>(out, pos);
-    out.push_back((uint8_t)(f[0].size() + 1));
-    out.push_back((uint8_t)mapq);
-    put_le<uint16_t>(out, 4680);  // bin: not used by the statistics
-    put_le<uint16_t>(out, (uint16_t)cigar.size());
-    put_le<uint16_t>(out, (uint16_t)flag);
-    put_le<int32_t>(out, (int32_t)seq.size());
-    put_le<int32_t>(out, nrid);
-    put_le<int32_t>(out, npos);
-    put_le<int32_t>(out, tlen);
-    out.insert(out.end(), f[0].begin(), f[0].end());
-    out.push_back(0);
-    for (uint32_t c : cigar) put_le<uint32_t>(out, c);
-    static const char nt16[] = "=ACMGRSVTWYHKDBN";
-    for (size_t i = 0; i < seq.size(); i += 2) {
-        auto code = [&](char ch) -> uint8_t {
-            const char* q = strchr(nt16, toupper((unsigned char)ch));
-            return q && ch ? (uint8_t)(q - nt16) : 15;
-        };
-        out.push_back((uint8_t)((code(seq[i]) << 4) | (i + 1 < seq.size() ? code(seq[i + 1]) : 0)));
-    }
-    if (f[10] == "*" || f[10].size() != seq.size()) out.insert(out.end(), seq.size(), 0xFF);
-    else for (char ch : f[10]) out.push_back((uint8_t)(ch - 33));
-    for (size_t t = 11; t < f.size(); ++t) {  // TAG:TYPE:VALUE
-        const std::string& a = f[t];
-        if (a.size() < 5 || a[2] != ':' || a[4] != ':') return false;
-        const char ty = a[3];
-        const std::string val = a.substr(5);
-        out.push_back((uint8_t)a[0]);
-        out.push_back((uint8_t)a[1]);
-        if (ty == 'A') { out.push_back('A'); out.push_back(val.empty() ? 0 : (uint8_t)val[0]); }
-        else if (ty == 'i') {  // the smallest BAM integer type that holds the value
-            const long long v = atoll(val.c_str());
-            if (v >= 0) {
-                if (v <= 255) { out.push_back('C'); out.push_back((uint8_t)v); }
-                else if (v <= 65535) { out.push_back('S'); put_le<uint16_t>(out, (uint16_t)v); }
-                else { out.push_back('I'); put_le<uint32_t>(out, (uint32_t)v); }
-            } else {
-                if (v >= -128) { out.push_back('c'); out.push_back((uint8_t)(int8_t)v); }
-                else if (v >= -32768) { out.push_back('s'); put_le<int16_t>(out, (int16_t)v); }
-                else { out.push_back('i'); put_le<int32_t>(out, (int32_t)v); }
-            }
-        } else if (ty == 'f') { out.push_back('f'); put_le<float>(out, (float)atof(val.c_str())); }
-        else if (ty == 'Z' || ty == 'H') { out.push_back((uint8_t)ty); out.insert(out.end(), val.begin(), val.end()); out.push_back(0); }
-        else if (ty == 'B') {
-            if (val.empty()) return false;
-            const char sub = val[0];
-            std::vector<std::string> items;
-            std::stringstream ss(val.size() > 2 ? val.substr(2) : std::string());
-            std::string item;
-            while (std::getline(ss, item, ',')) items.push_back(item);
-            out.push_back('B');
-            out.push_back((uint8_t)sub);
-            put_le<int32_t>(out, (int32_t)items.size());
-            for (const std::string& it : items) {
-                switch (sub) {
-                    case 'c': out.push_back((uint8_t)(int8_t)atoi(it.c_str())); break;
-                    case 'C': out.push_back((uint8_t)atoi(it.c_str())); break;
-                    case 's': put_le<int16_t>(out, (int16_t)atoi(it.c_str())); break;
-                    case 'S': put_le<uint16_t>(out, (uint16_t)atoi(it.c_str())); break;
-                    case 'i': put_le<int32_t>(out, (int32_t)atoll(it.c_str())); break;
-                    case 'I': put_le<uint32_t>(out, (uint32_t)atoll(it.c_str())); break;
-                    case 'f': put_le<float>(out, (float)atof(it.c_str())); break;
-                    default: return false;
-                }
-            }
-        } else return false;
-    }
-    const int32_t bs = (int32_t)(out.size() - start - 4);
-    memcpy(out.data() + start, &bs, 4);
-    return true;
-}
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -1206,65 +1072,73 @@ extern "C" int bqc_main(int argc, const char* const* argv) {
     auto t_start = std::chrono::steady_clock::now();
     if (!sam) return run_file(c, t_start);
     // ---- SAM text on stdin (src/bamqualcheck.cpp:252-260): one device ------------------------------------
-    std::vector<uint8_t> file;
-    std::string sam_pending;  // first alignment line, read while looking for the end of the header
-    bool sam_have_pending = false;
-    {
-        std::cerr << "Reading from stdin" << std::endl;  // src/CommandLineParser.hpp:96
-        std::string text, line;
-        while (std::getline(std::cin, line)) {
-            if (!line.empty() && line.back() == '\r') line.pop_back();
-            if (!line.empty() && line[0] == '@') { text += line; text += '\n'; continue; }
-            sam_pending = line;
-            sam_have_pending = true;
-            break;
+    // The header lines are read first; the alignment lines then go straight from read() into the staging buffers,
+    // each cut at its last line end (the partial line is carried into the next buffer), and are encoded on the GPU.
+    std::cerr << "Reading from stdin" << std::endl;  // src/CommandLineParser.hpp:96
+    auto read_some = [](char* dst, size_t cap, bool& eof) -> size_t {
+        for (;;) {
+            const ssize_t r = read(0, dst, cap);
+            if (r < 0 && errno == EINTR) continue;
+            if (r <= 0) { eof = true; return 0; }
+            return (size_t)r;
         }
-        file = sam_header_to_bam(text);
+    };
+    std::vector<char> head;
+    bool eof = false;
+    for (size_t line = 0;;) {   // until the first line that does not start with '@' (or the end of the input)
+        while (line < head.size() && head[line] == '@') {
+            const char* q = (const char*)memchr(head.data() + line, '\n', head.size() - line);
+            if (!q) break;
+            line = (size_t)(q - head.data()) + 1;
+        }
+        if ((line < head.size() && head[line] != '@') || eof) break;
+        const size_t at = head.size();
+        head.resize(at + (1u << 20));
+        head.resize(at + read_some(head.data() + at, 1u << 20, eof));
     }
     if (!probe_output(c)) return 1;
     bqc_bam_header hdr;
-    if (!bqc_parse_bam_header(file.data(), file.size(), &hdr)) {
+    size_t consumed = 0;
+    if (bqc_parse_sam_header(head.data(), head.size(), &hdr, &consumed)) {
         std::cerr << "ERROR: Could not open " << c.bam << " for reading.\n";
         return 1;
     }
     std::vector<uint8_t> main_chrom;
     bqc_engine* eng = make_engine(c, hdr, c.devices[0], main_chrom);
     if (!eng) return 1;
+    if (bqc_set_ref_names(eng, hdr.n_ref, hdr.ref_names)) { std::cerr << "ERROR: " << bqc_last_error(eng) << std::endl; return 1; }
     bqc_fasta* fa = bqc_fasta_open(c.ref.c_str());
     if (!fa) std::cerr << "ERROR: Could not open fasta file " << c.ref << std::endl;  // the reference continues too (:291)
     if (fa && !load_reference(eng, fa, hdr)) return 1;
     auto t_setup = std::chrono::steady_clock::now();
     int rc = 0;
     {
-        std::map<std::string, int32_t> ref_id;
-        for (int i = 0; i < hdr.n_ref; ++i) ref_id.insert({hdr.ref_names[i], i});  // first of duplicate names wins
-        std::vector<uint8_t> enc;
-        std::string line;
-        bool eof = false;
-        while (!eof && !rc) {
+        std::vector<char> carry(head.begin() + (ptrdiff_t)consumed, head.end());
+        head = std::vector<char>();
+        while (!rc) {
             void* pin;
             size_t cap;
             if (bqc_acquire_staging(eng, &pin, &cap)) { rc = 1; break; }
-            enc.clear();
-            const size_t room = cap > (1u << 20) ? cap - (1u << 20) : cap / 2;  // stop before a record could overflow the buffer
-            while (enc.size() < room) {
-                if (sam_have_pending) { line.swap(sam_pending); sam_have_pending = false; }
-                else if (!std::getline(std::cin, line)) { eof = true; break; }
-                if (!line.empty() && line.back() == '\r') line.pop_back();
-                if (line.empty()) continue;
-                if (!sam_line_to_bam(line, ref_id, enc)) {
-                    std::cerr << "ERROR: Could not read record from BAM File " << c.bam << "\n";
-                    rc = 1;
-                    break;
-                }
+            char* buf = (char*)pin;
+            if (carry.size() > cap) { std::cerr << "ERROR: SAM record larger than the staging buffer\n"; rc = 1; break; }
+            memcpy(buf, carry.data(), carry.size());
+            size_t filled = carry.size();
+            while (filled < cap && !eof) filled += read_some(buf + filled, cap - filled, eof);
+            size_t cut = filled;
+            if (!eof) {
+                while (cut > 0 && buf[cut - 1] != '\n') --cut;
+                if (cut == 0) { std::cerr << "ERROR: SAM record larger than the staging buffer\n"; rc = 1; break; }
             }
-            if (rc) break;
-            if (enc.size() > cap) { std::cerr << "ERROR: SAM record larger than the staging buffer\n"; rc = 1; break; }
-            memcpy(pin, enc.data(), enc.size());
-            if (bqc_submit_stream(eng, pin, enc.size(), eof ? 1 : 0)) rc = report_submit_error(eng, c);
+            carry.assign(buf + cut, buf + filled);
+            if (bqc_submit_sam(eng, buf, cut, eof ? 1 : 0)) {
+                bqc_sync(eng);   // the device's error word is final once the work in flight has run
+                report_finish_error(eng, c);
+                rc = 1;
+            }
+            if (eof) break;
         }
     }
-    if (!rc && bqc_finish(eng)) { report_finish_error(eng, c); rc = 1; }
+    if (!rc && bqc_finish(eng)) { bqc_sync(eng); report_finish_error(eng, c); rc = 1; }
     auto t_stats = std::chrono::steady_clock::now();
     if (!rc && bqc_write_bamqc(eng, hdr.sample_id, c.out.c_str())) {
         std::cerr << "ERROR: Could not open output file " << c.out << '\n';
@@ -1273,7 +1147,7 @@ extern "C" int bqc_main(int argc, const char* const* argv) {
     auto t_end = std::chrono::steady_clock::now();
     if (c.timing) {
         auto sec = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double>(b - a).count(); };
-        fprintf(stderr, "BAMQC_TIMING records=%llu setup_s=%.4f stats_s=%.4f write_s=%.4f total_s=%.4f threads=%d devices=1\n", (unsigned long long)bqc_records_seen(eng), sec(t_start, t_setup), sec(t_setup, t_stats), sec(t_stats, t_end), sec(t_start, t_end), c.threads);
+        fprintf(stderr, "BAMQC_TIMING records=%llu setup_s=%.4f stats_s=%.4f write_s=%.4f total_s=%.4f threads=%d devices=1 sam_host_lines=%llu\n", (unsigned long long)bqc_records_seen(eng), sec(t_start, t_setup), sec(t_setup, t_stats), sec(t_stats, t_end), sec(t_start, t_end), c.threads, (unsigned long long)bqc_sam_host_lines(eng));
     }
     if (fa) bqc_fasta_close(fa);
     bqc_destroy(eng);

@@ -559,4 +559,84 @@ int bqc_synth_write_bam(const char* path, const bqc_synth_params* p, const char*
     return 0;
 }
 
+// SAM text of the records (SAM/BAM specification 1.4 and 4.2): the header of bqc_synth_header_text, one line per
+// record.  B arrays, every integer type and f are written; the text encodes back to the same field values.
+int bqc_synth_write_sam(const char* path, const bqc_synth_params* p, const char* sample_id, const uint8_t* records, uint64_t n_bytes) {
+    FILE* f = fopen(path, "wb");
+    if (!f) return 1;
+    std::string line, head(bqc_synth_header_text(p, sample_id, nullptr, 0), '\0');
+    bqc_synth_header_text(p, sample_id, &head[0], head.size());
+    fwrite(head.data(), 1, head.size(), f);
+    static const char kOps[] = "MIDNSHP=X??????", kNt[] = "=ACMGRSVTWYHKDBN";
+    auto rd = [](const uint8_t* q, int n) { uint64_t v = 0; memcpy(&v, q, n); return v; };
+    auto ref = [&](int32_t id) { return id >= 0 && id < p->n_contigs ? std::string(p->names[id]) : std::string("*"); };
+    char num[64];
+    for (uint64_t o = 0; o + 4 <= n_bytes;) {
+        const uint32_t bs = (uint32_t)rd(records + o, 4);
+        const uint8_t* r = records + o + 4;
+        const uint8_t* end = r + bs;
+        o += 4 + (uint64_t)bs;
+        const int32_t rid = (int32_t)rd(r, 4), pos = (int32_t)rd(r + 4, 4), nrid = (int32_t)rd(r + 20, 4), npos = (int32_t)rd(r + 24, 4), tlen = (int32_t)rd(r + 28, 4);
+        const uint32_t lname = r[8], mapq = r[9], ncig = (uint32_t)rd(r + 12, 2), flag = (uint32_t)rd(r + 14, 2), lseq = (uint32_t)rd(r + 16, 4);
+        const uint8_t* q = r + 32;
+        line.assign((const char*)q, lname ? lname - 1 : 0);
+        q += lname;
+        snprintf(num, sizeof(num), "\t%u\t", flag);
+        line += num + ref(rid);
+        snprintf(num, sizeof(num), "\t%d\t%u\t", pos + 1, mapq);
+        line += num;
+        if (!ncig) line += '*';
+        for (uint32_t k = 0; k < ncig; ++k, q += 4) {
+            const uint32_t c = (uint32_t)rd(q, 4);
+            snprintf(num, sizeof(num), "%u%c", c >> 4, kOps[c & 15]);
+            line += num;
+        }
+        line += '\t';
+        line += nrid < 0 ? "*" : (nrid == rid ? "=" : ref(nrid));
+        snprintf(num, sizeof(num), "\t%d\t%d\t", npos + 1, tlen);
+        line += num;
+        if (!lseq) line += '*';
+        for (uint32_t k = 0; k < lseq; ++k) line += kNt[(q[k / 2] >> (k % 2 ? 0 : 4)) & 15];
+        q += (lseq + 1) / 2;
+        line += '\t';
+        if (!lseq || q[0] == 0xFF) line += '*';
+        else for (uint32_t k = 0; k < lseq; ++k) line += (char)(q[k] + 33);
+        q += lseq;
+        while (q + 3 <= end) {   // tags
+            const char t0 = (char)q[0], t1 = (char)q[1], ty = (char)q[2];
+            q += 3;
+            line += '\t'; line += t0; line += t1;
+            auto ival = [&](char t, const uint8_t* v) -> long long {
+                switch (t) {
+                    case 'c': return (int8_t)v[0]; case 'C': return v[0]; case 's': return (int16_t)rd(v, 2); case 'S': return (uint16_t)rd(v, 2);
+                    case 'i': return (int32_t)rd(v, 4); default: return (uint32_t)rd(v, 4);
+                }
+            };
+            auto isz = [](char t) { return t == 'c' || t == 'C' || t == 'A' ? 1 : t == 's' || t == 'S' ? 2 : 4; };
+            if (ty == 'A') { line += ":A:"; line += (char)q[0]; q += 1; }
+            else if (ty == 'Z' || ty == 'H') {
+                line += ty == 'Z' ? ":Z:" : ":H:";
+                const uint8_t* z = q;
+                while (z < end && *z) ++z;
+                line.append((const char*)q, z - q);
+                q = z + 1;
+            } else if (ty == 'f') { float x; memcpy(&x, q, 4); snprintf(num, sizeof(num), ":f:%.9g", x); line += num; q += 4; }
+            else if (ty == 'B') {
+                const char sub = (char)q[0];
+                const uint32_t cnt = (uint32_t)rd(q + 1, 4);
+                q += 5;
+                line += ":B:"; line += sub;
+                for (uint32_t k = 0; k < cnt; ++k, q += isz(sub)) {
+                    if (sub == 'f') { float x; memcpy(&x, q, 4); snprintf(num, sizeof(num), ",%.9g", x); }
+                    else snprintf(num, sizeof(num), ",%lld", ival(sub, q));
+                    line += num;
+                }
+            } else { snprintf(num, sizeof(num), ":i:%lld", ival(ty, q)); line += num; q += isz(ty); }
+        }
+        line += '\n';
+        if (fwrite(line.data(), 1, line.size(), f) != line.size()) { fclose(f); return 1; }
+    }
+    return fclose(f) ? 1 : 0;
+}
+
 }  // extern "C"

@@ -16,6 +16,29 @@ SCALAR_NAMES = ["supplementary", "duplicates", "QCfailed", "not_primary_alignmen
 DEFAULT_CHROMS = ",".join("chr%d" % i for i in range(1, 23))  # src/CommandLineParser.hpp:34
 
 
+BQC_ERR_ARG = 33
+
+
+def parse_sam_header(text):
+    """The '@' header lines at the front of SAM text -> (dict with text, ref_names, ref_lengths, lane_ids, sample_id,
+    offset of the first alignment line), through the same parser as a BAM header."""
+    b = text.encode() if isinstance(text, str) else bytes(text)
+    lib = _lib.load_library()
+    h = _lib.bqc_bam_header()
+    used = ctypes.c_size_t()
+    rc = lib.bqc_parse_sam_header(b, len(b), ctypes.byref(h), ctypes.byref(used))
+    if rc:
+        raise BamQCError(rc, "malformed SAM header")
+    try:
+        out = {"text": h.text.decode(), "ref_names": [h.ref_names[i].decode() for i in range(h.n_ref)],
+               "ref_lengths": [int(h.ref_lengths[i]) for i in range(h.n_ref)],
+               "lane_ids": [h.lane_ids[i].decode() for i in range(h.n_lanes)],
+               "sample_id": h.sample_id.decode() if h.sample_id else ""}
+    finally:
+        lib.bqc_free_bam_header(ctypes.byref(h))
+    return out, used.value
+
+
 class BamQCError(RuntimeError):
     def __init__(self, code, message, record=None):
         super().__init__(f"[bqc error {code}] {message}")
@@ -77,6 +100,7 @@ class Engine:
             raise BamQCError(rc, self.lib.bqc_last_error(None).decode())
         self.handle = h
         self.device = device
+        self._sam_refs_set = False
 
     # ---- lifetime ---------------------------------------------------------------------------------
     def close(self):
@@ -134,6 +158,37 @@ class Engine:
         a = _as_u8(data)
         self._check(self.lib.bqc_submit_bgzf(self.handle, a.ctypes.data if a.size else None, a.size, skip, 1 if last else 0))
 
+    def _sam_refs(self):  # bqc_set_ref_names once, before the first SAM text
+        if not self._sam_refs_set:
+            names = (ctypes.c_char_p * max(1, len(self.ref_names)))(*[r.encode() for r in self.ref_names])
+            self._check(self.lib.bqc_set_ref_names(self.handle, len(self.ref_names), names))
+            self._sam_refs_set = True
+
+    def submit_sam(self, data, last=False):
+        """SAM alignment lines (no header lines), ending at a line end unless `last`; encoded to BAM records on the
+        device.  RNAME/RNEXT are looked up in `ref_names`."""
+        self._sam_refs()
+        a = _as_u8(data.encode() if isinstance(data, str) else data)
+        self._check(self.lib.bqc_submit_sam(self.handle, a.ctypes.data if a.size else None, a.size, 1 if last else 0))
+
+    def sam_to_bam(self, text):
+        """The BAM records (block_size included) that submit_sam counts for `text`, as bytes."""
+        self._sam_refs()
+        a = _as_u8(text.encode() if isinstance(text, str) else text)
+        out = np.empty(2 * a.size + 64, dtype=np.uint8)
+        nb, nr = ctypes.c_uint64(), ctypes.c_uint64()
+        rc = self.lib.bqc_sam_to_bam(self.handle, a.ctypes.data if a.size else None, a.size, out.ctypes.data, out.size, ctypes.byref(nb), ctypes.byref(nr))
+        if rc == BQC_ERR_ARG:   # a host-encoded submission (B arrays) may need more than twice the text
+            out = np.empty(8 * a.size + 64, dtype=np.uint8)
+            rc = self.lib.bqc_sam_to_bam(self.handle, a.ctypes.data if a.size else None, a.size, out.ctypes.data, out.size, ctypes.byref(nb), ctypes.byref(nr))
+        self._check(rc)
+        return out[:nb.value].tobytes()
+
+    @property
+    def sam_host_lines(self):
+        """Non-empty SAM lines that went through the host encoder (submissions outside the device grammar)."""
+        return int(self.lib.bqc_sam_host_lines(self.handle))
+
     @property
     def frames_repaired(self):
         return int(self.lib.bqc_frames_repaired(self.handle))
@@ -179,7 +234,7 @@ class Engine:
         n = (ctypes.c_uint64 * 12)()
         self._check(self.lib.bqc_profile_read(self.handle, ms, n))
         names = ["k_stats", "k_eightmer", "k_sketch", "k_cov", "merge", "host_framing", "host_scan_pass1", "host_scan_pass2",
-                 "k_inflate", "k_frame", "_10", "_11"]
+                 "k_inflate", "k_frame", "k_sam", "_11"]
         return {names[i]: (float(ms[i]), int(n[i])) for i in range(12)}
 
     # ---- multi-GPU merge ----------------------------------------------------------------------------

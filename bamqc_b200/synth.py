@@ -128,6 +128,14 @@ def header_text(genome, lib_, sample_id="S1"):
     return buf.raw[:n].decode()
 
 
+def write_sam(path, genome, lib_, records, n_bytes, sample_id="S1"):
+    """SAM text of the records (header + one line per record), written by the C generator."""
+    L = _lib.load_synth()
+    p = _Params(genome, lib_)
+    if L.bqc_synth_write_sam(str(path).encode(), ctypes.byref(p.c), sample_id.encode(), records.ctypes.data, n_bytes):
+        raise IOError(path)
+
+
 def write_bam(path, genome, lib_, records, n_bytes, sample_id="S1", level=-1):
     """level -1: raw uncompressed BAM stream; 0..9: BGZF."""
     L = _lib.load_synth()

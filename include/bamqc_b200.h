@@ -110,6 +110,24 @@ int bqc_submit_bgzf(bqc_engine* e, const void* data, size_t n_bytes, size_t skip
 int bqc_stream_unknown_start(bqc_engine* e);
 int bqc_stream_skipped(bqc_engine* e, uint64_t* skipped);   /* 0: known; -1: the first submission has not been framed yet (poll; may be
                                                                called from another thread); > 0: the engine's error code */
+/* ---- SAM text -------------------------------------------------------------------------------------
+ * The @SQ names in header order (n == cfg.n_ref), for RNAME/RNEXT: the first of duplicate names wins, an unknown name
+ * is -1.  Call it before the first SAM submission. */
+int bqc_set_ref_names(bqc_engine* e, int32_t n, const char* const* names);
+/* Submit SAM alignment lines (no '@' header lines), asynchronously like bqc_submit_stream; pinned or pageable memory,
+ * at most the staging capacity.  The text must end at a line end unless `last` is set (then a final line without
+ * '\n' counts); otherwise BQC_ERR_ARG.  Empty lines are skipped and a trailing '\r' is dropped.  The lines are encoded
+ * to BAM records on the device; a submission holding a line outside the device's grammar (B arrays, for one; see
+ * csrc/sam_parse.h) is encoded on the host instead, with the same records.  A line the encoder rejects is
+ * BQC_ERR_BAD_RECORD at that line's record index; the records in front of it still run. */
+int bqc_submit_sam(bqc_engine* e, const void* text, size_t n, int last);
+/* The BAM records (block_size included, back to back) that bqc_submit_sam would count for text[0..n), copied into
+ * out[0..cap).  Synchronous; counts nothing.  On BQC_ERR_BAD_RECORD *n_records is the index of the rejected line's
+ * record and out holds the records in front of it. */
+int bqc_sam_to_bam(bqc_engine* e, const void* text, size_t n, uint8_t* out, uint64_t cap, uint64_t* n_bytes, uint64_t* n_records);
+/* Non-empty lines encoded on the host so far (submissions that fell back, by bqc_submit_sam or bqc_sam_to_bam). */
+uint64_t bqc_sam_host_lines(bqc_engine* e);
+
 /* Number of stream buffers whose speculative framing failed verification and were re-framed sequentially. */
 uint64_t bqc_frames_repaired(bqc_engine* e);
 /* Records submitted so far (waits for the submissions in flight to be framed). */
@@ -133,7 +151,7 @@ int bqc_get_error(bqc_engine* e, bqc_error_info* out); /* sticky device/host err
 /* Optional device timing of each kernel family with CUDA events on the compute stream.
  * bqc_profile_read: milliseconds and launch-group counts accumulated since the previous read, per family:
  * 0 k_stats, 1 k_eightmer, 2 k_sketch, 3 coverage kernels, 4 merge/export, 5-6 host framing / header
- * pre-pass of host-framed submissions (wall clock), 7 unused, 8 k_inflate, 9 framing kernels. */
+ * pre-pass of host-framed submissions (wall clock), 7 unused, 8 k_inflate, 9 framing kernels, 10 SAM text kernels. */
 void bqc_profile_enable(bqc_engine* e, int on);
 int bqc_profile_read(bqc_engine* e, double ms_out[12], uint64_t n_out[12]);
 
@@ -250,6 +268,9 @@ typedef struct bqc_bam_header {
     char* sample_id;     /* last @RG SM */
 } bqc_bam_header;
 size_t bqc_parse_bam_header(const uint8_t* data, size_t n, bqc_bam_header* out);
+/* Parse the header lines ('@' lines) at the front of SAM text into the same structure; *consumed is the length of the
+ * header lines (the offset of the first alignment line).  0 on success, BQC_ERR_ARG on a malformed header. */
+int bqc_parse_sam_header(const char* text, size_t n, bqc_bam_header* out, size_t* consumed);
 void bqc_free_bam_header(bqc_bam_header* h);
 /* Find record boundaries in [data, data+n): fills offsets (cap entries) with the start of each whole
  * record plus the end of the last whole one; returns the number of whole records. */

@@ -67,6 +67,9 @@ int bqc_synth_records(const bqc_synth_params* p, uint8_t* out, uint64_t out_cap,
 int bqc_synth_write_bam(const char* path, const bqc_synth_params* p, const char* sample_id,
                         const uint8_t* records, uint64_t n_bytes, int compress_level);
 
+/* Write a SAM text file: the header of bqc_synth_header_text and one alignment line per record. Returns 0 on success. */
+int bqc_synth_write_sam(const char* path, const bqc_synth_params* p, const char* sample_id, const uint8_t* records, uint64_t n_bytes);
+
 /* BGZF-compress an arbitrary byte stream into memory (for end-to-end inflate benchmarks).
  * Returns compressed size, or 0 if cap is too small. */
 uint64_t bqc_synth_bgzf_compress(const uint8_t* in, uint64_t n, int level, uint8_t* out, uint64_t cap);
